@@ -140,6 +140,7 @@ int kite_jac_sparsity(int model_kind, int has_arm, int wrt_u, int* row_out, int*
  *   traj_d NULL or [N/save_every][13][ld]: state after every save_every-th step
  *   y_d NULL or [N][13]: shared measurement log; if given, cost_d[ld] receives the identification cost
  *        (1/N) sum_k sum_c Q_c (y[k][c] - x_c(k+1))^2   (kite_identification_test.cpp:193-205)
+ *        which has no value for N = 0: y_d with N = 0 is rejected with KITE_ERR_ARG (also by kite_rk4_rollout_host)
  *   status_d NULL or int32[ld]: 0 = ok, 1 = non-finite state reached
  *   index0: global index of trajectory 0 of this call (only used by KITE_U_SYNTH; sharding-invariant inputs) */
 int kite_rk4_rollout(kite_ctx* ctx, long B, long ld, long N, double h, const double* x0_d, const double* u_d, int u_mode,

@@ -254,6 +254,7 @@ int kite_rk4_rollout(kite_ctx* ctx, long B, long ld, long N, double h, const dou
     if (u_mode != KITE_U_SYNTH && !u_d && !rigid) return fail(ctx, KITE_ERR_ARG, "kite_rk4_rollout: u_d is null");
     if (rigid && (p_d || u_mode == KITE_U_SYNTH)) return fail(ctx, KITE_ERR_STATE, "kite_rk4_rollout: not valid for rigid body");
     if ((y_d != nullptr) != (cost_d != nullptr)) return fail(ctx, KITE_ERR_ARG, "kite_rk4_rollout: y_d and cost_d go together");
+    if (y_d && N == 0) return fail(ctx, KITE_ERR_ARG, "kite_rk4_rollout: the fitting cost averages over the steps and needs N > 0");
     if (traj_d && save_every <= 0) return fail(ctx, KITE_ERR_ARG, "kite_rk4_rollout: save_every must be > 0");
     if (N >= (1L << 31) || save_every >= (1L << 31)) return fail(ctx, KITE_ERR_ARG, "kite_rk4_rollout: N and save_every must be below 2^31");
     if (B == 0) return KITE_OK;
