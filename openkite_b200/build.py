@@ -29,12 +29,11 @@ def _newest_header():
     return t
 
 
-def _compile(unit, verbose, obj_dir=None, extra=()):
-    obj_dir = obj_dir or OBJ
+def _compile(unit, verbose):
     src = os.path.join(CSRC, unit + ".cu")
-    obj = os.path.join(obj_dir, unit + ".o")
-    log = os.path.join(obj_dir, unit + ".ptxas.log")
-    cmd = ["nvcc", *NVCC_FLAGS, *extra, "-c", src, "-o", obj]
+    obj = os.path.join(OBJ, unit + ".o")
+    log = os.path.join(OBJ, unit + ".ptxas.log")
+    cmd = ["nvcc", *NVCC_FLAGS, "-c", src, "-o", obj]
     r = subprocess.run(cmd, capture_output=True, text=True)
     with open(log, "w") as fh:
         fh.write(r.stdout + r.stderr)
@@ -84,21 +83,6 @@ def build_casadi_shim(force=False):
     return LIB_CASADI
 
 
-def build_variant(tag, extra_flags):
-    """Developer experiments only: full rebuild with extra -D flags into openkite_b200/_variants/<tag>/libkite_b200.so
-    (scripts/gpu_sweep_rollout.py loads such a library by path).  The product library is always LIB."""
-    vdir = os.path.join(HERE, "_variants", tag)
-    os.makedirs(vdir, exist_ok=True)
-    with ThreadPoolExecutor(max_workers=8) as ex:
-        objs = list(ex.map(lambda u: _compile(u, False, vdir, tuple(extra_flags)), UNITS))
-    lib = os.path.join(vdir, "libkite_b200.so")
-    r = subprocess.run(["nvcc", "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", lib, *objs, "-ldl"],
-                       capture_output=True, text=True)
-    if r.returncode != 0:
-        raise RuntimeError("link failed:\n" + r.stdout + r.stderr)
-    return lib
-
-
 def resource_report():
     """(kernel, registers, spill bytes) parsed from the saved ptxas logs."""
     import re
@@ -115,10 +99,6 @@ def resource_report():
 
 
 if __name__ == "__main__":
-    if "--variant" in sys.argv:
-        k = sys.argv.index("--variant")
-        print(build_variant(sys.argv[k + 1], sys.argv[k + 2:]))
-        sys.exit(0)
     lib = build(force="--force" in sys.argv, verbose="--verbose" in sys.argv)
     print(lib)
     for name, regs, stack, sst, sld in resource_report():

@@ -7,7 +7,6 @@
 
 #include <algorithm>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -415,9 +414,8 @@ static int sens_impl(kite_ctx* ctx, long B, long ld, long N, double h, const dou
     a.status = ctx->status_out;
     if (a.status) CK(cudaMemsetAsync(a.status, 0, sizeof(int32_t) * (size_t)B, ctx->stream));      // the kernel ORs flags in
     // [Phi | Gamma] leave through TMA tensor stores when the output layout allows it (16-byte aligned base and pitch:
-    // an even ld; an even B); KITE_SENS_DIRECT_STORES=1 forces the direct-store kernel (developer comparison switch)
-    static const bool direct = getenv("KITE_SENS_DIRECT_STORES") && getenv("KITE_SENS_DIRECT_STORES")[0] == '1';
-    const bool tma_out = !rigid && !direct && sens_make_tensor_map(&a.tmPhi, Phi, B, ld, 169, N) &&
+    // an even ld; an even B)
+    const bool tma_out = !rigid && sens_make_tensor_map(&a.tmPhi, Phi, B, ld, 169, N) &&
                          sens_make_tensor_map(&a.tmGam, Gamma, B, ld, 39, N);
     launch_sens_fused(a, rigid, ctx->K.has_arm != 0, tma_out, ctx->stream);
     LAUNCH_CHECK("k_sens_fused");

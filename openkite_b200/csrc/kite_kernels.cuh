@@ -114,33 +114,10 @@ struct RolloutArgs {
     long index0;
 };
 
-// load flavour of the per-step control stream (read once): __ldg, or ld.global.L1::no_allocate to keep the stream out of L1
-__device__ __forceinline__ double ld_noalloc(const double* p) {
-    double v;
-    asm volatile("ld.global.L1::no_allocate.f64 %0, [%1];" : "=d"(v) : "l"(p));
-    return v;
-}
-#ifndef KITE_LDU
-#define KITE_LDU __ldg
-#endif
-#ifndef KITE_ROLLOUT_BLOCK
-#define KITE_ROLLOUT_BLOCK 128
-#endif
-constexpr int ROLLOUT_BLOCK = KITE_ROLLOUT_BLOCK;
-#ifndef KITE_ROLLOUT_SMEM_STATE
-#define KITE_ROLLOUT_SMEM_STATE 0     // 1: base state + tableau accumulator in shared memory, 4 CTAs per SM at 128 registers
-#endif
-#ifndef KITE_ROLLOUT_CTAS
-#define KITE_ROLLOUT_CTAS (KITE_ROLLOUT_SMEM_STATE ? 4 : 3)
-#endif
-#ifdef KITE_ROLLOUT_MAXNREG          // experiments: cap registers directly (occupancy between the launch-bounds steps)
-#define KITE_ROLLOUT_ATTR __maxnreg__(KITE_ROLLOUT_MAXNREG)
-#else
-#define KITE_ROLLOUT_ATTR __launch_bounds__(ROLLOUT_BLOCK, KITE_ROLLOUT_CTAS)
-#endif
-// dynamic shared memory of a rollout CTA: [per-trajectory coefficients (PERCOEF)][x 13 x BLOCK][acc 13 x BLOCK (SMEM_STATE)]
+constexpr int ROLLOUT_BLOCK = 128;
+// dynamic shared memory of a rollout CTA: the per-trajectory coefficients (PERCOEF)
 constexpr size_t rollout_smem_bytes(bool percoef) {
-    return (percoef ? sizeof(AeroCoef) * ROLLOUT_BLOCK : 0) + (KITE_ROLLOUT_SMEM_STATE ? sizeof(double) * 26 * ROLLOUT_BLOCK : 0);
+    return percoef ? sizeof(AeroCoef) * ROLLOUT_BLOCK : 0;
 }
 
 // Per-warp scratch lines that are written and re-read within microseconds (stage states of the sensitivity kernel, Jacobian
@@ -171,10 +148,10 @@ __device__ __forceinline__ long fresh_thread_index() {
 }
 
 template <int UMODE, bool RIGID, class AC>
-__device__ __forceinline__ void rollout_body(const RolloutArgs& a, double (&x)[13], double (&u)[3], const AC& A, double* st_sh);
+__device__ __forceinline__ void rollout_body(const RolloutArgs& a, double (&x)[13], double (&u)[3], const AC& A);
 
 template <int UMODE, bool RIGID, bool PERCOEF>
-__global__ void KITE_ROLLOUT_ATTR k_rk4_rollout(const __grid_constant__ RolloutArgs a) {
+__global__ void __launch_bounds__(ROLLOUT_BLOCK, 3) k_rk4_rollout(const __grid_constant__ RolloutArgs a) {
     // per-trajectory aero coefficients (identification sweeps) live in shared memory, one 21-double record per thread
     // (odd stride: conflict free): 42 registers the RHS cannot spare (they spilled: 96 B / 80 B per thread in round 1)
     extern __shared__ __align__(16) unsigned char rollout_smem[];
@@ -194,20 +171,13 @@ __global__ void KITE_ROLLOUT_ATTR k_rk4_rollout(const __grid_constant__ RolloutA
             reinterpret_cast<AeroCoef*>(rollout_smem)[threadIdx.x] = At;
         }
     }
-    double* const st_sh = reinterpret_cast<double*>(rollout_smem + (PERCOEF ? sizeof(AeroCoef) * ROLLOUT_BLOCK : 0)) + threadIdx.x;
-    if constexpr (PERCOEF) rollout_body<UMODE, RIGID>(a, x, u, reinterpret_cast<const volatile AeroCoef*>(rollout_smem)[threadIdx.x], st_sh);
-    else rollout_body<UMODE, RIGID>(a, x, u, a.K.A, st_sh);
+    if constexpr (PERCOEF) rollout_body<UMODE, RIGID>(a, x, u, reinterpret_cast<const volatile AeroCoef*>(rollout_smem)[threadIdx.x]);
+    else rollout_body<UMODE, RIGID>(a, x, u, a.K.A);
 }
 
 template <int UMODE, bool RIGID, class AC>
-__device__ __forceinline__ void rollout_body(const RolloutArgs& a, double (&x)[13], double (&u)[3], const AC& A, double* st_sh) {
+__device__ __forceinline__ void rollout_body(const RolloutArgs& a, double (&x)[13], double (&u)[3], const AC& A) {
     const long i = fresh_thread_index();
-#if KITE_ROLLOUT_SMEM_STATE
-    double* const xs = st_sh;                                        // x[c] at xs[c * BLOCK], acc[c] at as[c * BLOCK]
-    double* const as = st_sh + 13 * ROLLOUT_BLOCK;
-#pragma unroll
-    for (int c = 0; c < 13; ++c) xs[c * ROLLOUT_BLOCK] = x[c];
-#endif
 
     // Controls.  KITE_U_PER_STEP streams 24 B per state-step from HBM; the loads of step k + 1 are issued at the top of step k
     // (below) and have a whole step (~4 us) to land, so nothing else is needed: the L2 prefetch two steps ahead that round 1
@@ -223,7 +193,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, double (&x)[1
             for (int c = 0; c < 3; ++c) uu[c] = __ldg(a.u + (long)c * a.ld + i);
         } else if constexpr (UMODE == 1) {
 #pragma unroll
-            for (int c = 0; c < 3; ++c) uu[c] = KITE_LDU(up + (long)c * a.ld);
+            for (int c = 0; c < 3; ++c) uu[c] = __ldg(up + (long)c * a.ld);
         } else if constexpr (UMODE == 2) {
 #pragma unroll
             for (int c = 0; c < 3; ++c) uu[c] = __ldg(up + c);
@@ -255,15 +225,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, double (&x)[1
         } else if constexpr (UMODE == 3) {
             load_u(k, u);
         }
-#if KITE_ROLLOUT_SMEM_STATE
-        rk4_step_sm<RIGID, ROLLOUT_BLOCK>(a.K, A, xs, as, u, a.rk);
-        if (yp || (a.traj && k + 1 == next_save)) {
-#pragma unroll
-            for (int c = 0; c < 13; ++c) x[c] = xs[c * ROLLOUT_BLOCK];
-        }
-#else
         rk4_step<RIGID>(a.K, A, x, u, a.rk);
-#endif
         if (yp) {                                   // uniform branch: identification cost fused into the rollout
             double e = 0.0;
 #pragma unroll
@@ -282,10 +244,6 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& a, double (&x)[1
         }
     }
     const long io = fresh_thread_index();
-#if KITE_ROLLOUT_SMEM_STATE
-#pragma unroll
-    for (int c = 0; c < 13; ++c) x[c] = xs[c * ROLLOUT_BLOCK];
-#endif
 #pragma unroll
     for (int c = 0; c < 13; ++c) a.xf[(long)c * a.ld + io] = x[c];
     if (a.y) a.cost[io] = cost * (1.0 / (double)a.N);
@@ -406,10 +364,8 @@ static_assert(make_sens_tab().jx[5][12] == SENS_SLOTS - 1, "sens slot numbering"
 static_assert(make_sens_tab().jx[10][3] == make_sens_tab().jx[12][5] && make_sens_tab().jx[9][3] == make_sens_tab().jx[11][5],
               "shared quaternion-rate slots");
 
-#ifndef KITE_SF_WARPS
-#define KITE_SF_WARPS 8                        // 8 warps x 255 registers = the whole register file, 2 warps per scheduler
-#endif
-constexpr int SF_WARPS = KITE_SF_WARPS;        // upper bound of warps per CTA (one CTA per SM)
+// upper bound of warps per CTA (one CTA per SM): 8 warps x 255 registers = the whole register file, 2 warps per scheduler
+constexpr int SF_WARPS = 8;
 constexpr size_t SF_SMEM_MAX = 227 * 1024;
 constexpr long SF_SCRATCH_PER_WARP = 4L * 16 * 32;      // doubles: [stage][x(13) | u(3)][32 units]
 template <bool ARM> struct SfCfg {
@@ -593,7 +549,6 @@ __global__ void __launch_bounds__(SfCfg<ARM>::WARPS * 32, 1) k_sens_fused(const 
 #pragma unroll 1
         for (int r = 0; r < 4; ++r) {
             // ---------------- step 2: lane = (unit, stage), four stage Jacobians of 8 units -> shared tile ----------
-#ifndef KITE_SF_SKIP_A      // (developer timing switch: skip one phase to profile the other alone; results are garbage)
             {
                 const int u8 = lane & 7, s = lane >> 3;
                 double xt[13], u[3], k[13];
@@ -609,9 +564,7 @@ __global__ void __launch_bounds__(SfCfg<ARM>::WARPS * 32, 1) k_sens_fused(const 
                 }
                 model_eval<RIGID, true>(a.K, a.K.A, xt, u, k, sink);
             }
-#endif
             __syncwarp();                               // the tile is complete and visible to all lanes
-#ifndef KITE_SF_SKIP_B
             // ---------------- phase B: 8 lanes = unit, 4 units per pass ---------------------------------------------
             double D[2][16], N0[13], N1[13], A0[13], A1[13];   // D[.][13..15]: the control part of the seed (constant)
 #pragma unroll
@@ -727,7 +680,6 @@ __global__ void __launch_bounds__(SfCfg<ARM>::WARPS * 32, 1) k_sens_fused(const 
                     }
                 }
             }
-#endif
             __syncwarp();                               // every lane is done reading the tile before the next round
         }
         item = item_next;
@@ -926,9 +878,6 @@ struct EkfTmaArgs {
     EkfArgs e;
     double* Jw;                       // scratch: [resident warp][4 rounds][NS slots][8 filters]
 };
-#ifndef KITE_EKF_NOTMA
-#define KITE_EKF_NOTMA 0        // developer timing switch (results are garbage): 1 = no covariance traffic at all, 2 = no loads, stores kept
-#endif
 template <bool ARM> struct EtCfg {
     static constexpr int NS = ARM ? SENS_SLOTS : SENS_SLOTS_NOARM - 7;          // state-Jacobian slots (no Ju)
     static constexpr int TILE_D = NS * 8;                                         // doubles per round tile [slot][8 filters]
@@ -992,7 +941,7 @@ __global__ void __launch_bounds__(EtCfg<ARM>::WARPS * 32, 1) k_ekf_predict_tma(c
 
     // box of the warp's round `t` (filters first .. first + 7) -> buffer t & 1, one TMA tensor load issued by lane 0
     auto issue_load = [&](unsigned t, long first) {
-        if (!KITE_EKF_NOTMA && lane == 0) {
+        if (lane == 0) {
             const unsigned bar = smem_u32(bars + (t & 1));
             asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(bar), "r"(C::BOX_BYTES) : "memory");
             asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
@@ -1066,7 +1015,7 @@ __global__ void __launch_bounds__(EtCfg<ARM>::WARPS * 32, 1) k_ekf_predict_tma(c
                 else { mbar_wait(bars + 2, tile_ph0); tile_ph0 ^= 1; }
             }
             unsigned char* const box = wb + (t & 1) * C::BOX;
-            if (!KITE_EKF_NOTMA) mbar_wait(bars + (t & 1), (t >> 1) & 1);
+            mbar_wait(bars + (t & 1), (t >> 1) & 1);
             // ---------------- phase B: 8 lanes = filter, 2 passes of 4 filters ---------------------------------
             // Box entry (row, col) of this lane's filter sits at box + (row * 13 + col) * 64 + filter * 8 with the TMA's 64-byte
             // swizzle (16-byte chunk index ^= address bits 7..8).  The swizzled address is computed from the absolute shared
@@ -1118,7 +1067,7 @@ __global__ void __launch_bounds__(EtCfg<ARM>::WARPS * 32, 1) k_ekf_predict_tma(c
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             __syncwarp();                           // every lane is done with the tile and the box of this round
             if (r < 2) issue_tile(t + 2, r + 2);    // this round's tile buffer is free: the tile of round r + 2 lands a round ahead
-            if (KITE_EKF_NOTMA != 1 && lane == 0) {                            // filters >= B are clipped by the tensor map
+            if (lane == 0) {                            // filters >= B are clipped by the tensor map
                 asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%1, %2, %3}], [%4];"
                              :: "l"(reinterpret_cast<unsigned long long>(&ta.tmPn)), "r"((int)(g * 32 + r * 8)), "r"(0), "r"(0),
                                 "r"(smem_u32(box)) : "memory");
@@ -1152,11 +1101,8 @@ struct EkfUpdArgs {
     const double* V;         // device [49]
     int32_t* status;         // [ld] per-filter flag (non-finite updated state: singular innovation covariance) or null
 };
-#ifndef KITE_EKFU_COLS
-#define KITE_EKFU_COLS 2
-#endif
 constexpr int EKFU_BLOCK = 128;
-constexpr int EKFU_COLS = KITE_EKFU_COLS;       // covariance columns per pass of the update
+constexpr int EKFU_COLS = 2;         // covariance columns per pass of the update
 constexpr int EKFU_KUNROLL = 4;      // rows of K in flight: 28 loads instead of 7 between dependent DRAM round trips (0.88 -> 0.81 ms)
 template <int DUMMY = 0>
 __global__ void __launch_bounds__(EKFU_BLOCK, 2) k_ekf_update(const __grid_constant__ EkfUpdArgs a) {

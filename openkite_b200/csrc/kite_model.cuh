@@ -19,10 +19,6 @@
 
 #include "kite_math.cuh"
 
-#ifndef KITE_CB_DIRECT
-#define KITE_CB_DIRECT 0
-#endif
-
 namespace kite {
 
 // Derived aerodynamic coefficients (from the 21 raw coefficients, kite.cpp:571-572 order).
@@ -168,30 +164,20 @@ __device__ __forceinline__ void kite_eval_c(const KiteConsts& K, const AC& A, co
     const double V = is_pos(V2) ? V2 * rV : 0.0;              // v = 0 is a legal state of the standard model
     const double iVe = fast_rcp(V + K.eps);
     const double sb = v[1] * iVe;                             // sin(sideslip)
-#if KITE_CB_DIRECT
-    // cos(sideslip) = sqrt(1 - sb^2) = sqrt((V + eps)^2 - v1^2) / (V + eps), and (V + eps)^2 - v1^2 = v0^2 + v2^2 + eps (2 V + eps):
-    // no cancellation near |sb| = 1 and the square root no longer waits for the reciprocal (shorter dependency chain)
-    const double w2 = fma(K.eps, fma(2.0, V, K.eps), fma(v[0], v[0], v[2] * v[2]));
-    const double rw = fast_rsqrt(w2);
-    const double sw = is_pos(w2) ? w2 * rw : 0.0;
-    const double cb = sw * iVe;                               // cos(sideslip) >= 0
-    const double rcb = (V + K.eps) * rw;                      // 1/cos(sideslip)
-#else
     const double c2 = fma(-sb, sb, 1.0);
     const double rcb = fast_rsqrt(c2);                        // 1/cos(sideslip)
     const double cb = is_pos(c2) ? c2 * rcb : 0.0;            // cos(sideslip) >= 0
-#endif
     const double xe = v[0] + K.eps;
     const double irho = fast_rsqrt(fma(xe, xe, v[2] * v[2]));
     const double ca = xe * irho, sa = v[2] * irho;            // cos/sin(angle of attack)
     // both angles from their (sin, cos) pairs, branch free for any sideslip and any angle of attack (all four
     // quadrants): two interleaved polynomial chains, no division, no libm, no warp divergence (kite_math.cuh)
-    // Angles: table + short series in every kernel (KITE_ANGLE_TABLE, kite_math.cuh: config 2 +1.6 %).  Exponential of the
+    // Angles: table + short series in every kernel (asin_sc<true>, kite_math.cuh: config 2 +1.6 %).  Exponential of the
     // tether logistic: the 2^(j/32) table form only where the coefficients come from shared memory (identification sweeps:
     // +1.6 % on top of the angle table there, -0.5 % on the config-2 kernel: profiles/r2e_sweep_tables.log, r2r_sweep.log)
     constexpr bool TAB = exp_table_for<AC>::value;
-    const double ss = asin_sc<TAB || (KITE_ANGLE_TABLE != 0)>(sb, cb);
-    const double aoa = atan2_sc<TAB || (KITE_ANGLE_TABLE != 0)>(sa, ca);
+    const double ss = asin_sc<true>(sb, cb);
+    const double aoa = atan2_sc<true>(sa, ca);
     const double qS = K.cqS * V2;
 
     // ---- aerodynamic force in the wind frame, rotated to body ---------------------------
@@ -231,7 +217,7 @@ __device__ __forceinline__ void kite_eval_c(const KiteConsts& K, const AC& A, co
     const double d = d2 * id;
     const double n[3] = {r[0] * id, r[1] * id, r[2] * id};
     const double e = d - K.Lt;
-    const double H = fast_logistic<TAB || (KITE_EXP_TABLE != 0)>(4.0 * e);                  // K/(1+exp(-4x)), kitemath.cpp:31-34
+    const double H = fast_logistic<TAB>(4.0 * e);                   // K/(1+exp(-4x)), kitemath.cpp:31-34
     const double nv = fma(n[0], vi[0], fma(n[1], vi[1], n[2] * vi[2]));
     const double tens = fma(K.Ks, e, K.Kd * nv);
     const double tau = tens * H;
@@ -560,9 +546,6 @@ __device__ __forceinline__ void model_eval_c(const KiteConsts& K, const AC& A, c
     else kite_eval_c<JAC>(K, A, x, uc, f, sink);
 }
 
-#ifndef KITE_CB_DIRECT
-#define KITE_CB_DIRECT 0
-#endif
 // One classical RK4 step in registers (kitemath.cpp:36-51): x <- x + h/6 (k1 + 2 k2 + 2 k3 + k4).
 // Tableau of the classical RK4 step for one step size, filled on the host and read from the kernel's constant bank:
 //   an[st] = offset of the NEXT stage (h/2, h/2, h, -), w[st] = weight (1, 2, 2, 1), h6 = h / 6.
@@ -606,42 +589,6 @@ __device__ __forceinline__ void rk4_step(const KiteConsts& K, const AC& A, doubl
     }
 #pragma unroll
     for (int i = 0; i < 13; ++i) x[i] = fma(rk.h6, acc[i], x[i]);
-}
-
-// The same step with the base state x and the tableau accumulator in SHARED memory (this thread's column, stride ST doubles;
-// volatile: read at the point of use, never cached in registers): 52 registers less across the RHS, which is what a fourth
-// CTA per SM needs (k_rk4_rollout, KITE_ROLLOUT_SMEM_STATE).
-template <bool RIGID, int ST, class AC>
-__device__ __forceinline__ void rk4_step_sm(const KiteConsts& K, const AC& A, double* xs, double* as,
-                                            const double (&u)[3], const RkTab& rk) {
-    NoSink ns;
-    double k[13], xt[13];
-#pragma unroll
-    for (int i = 0; i < 13; ++i) xt[i] = xs[i * ST];
-    const CtrlTerms uc = ctrl_terms(K, A, u);
-#pragma unroll 1
-    for (int st = 0; st < 4; ++st) {
-        model_eval_c<RIGID, false>(K, A, xt, uc, k, ns);
-        // the pointers are laundered once per stage: the loads below may be scheduled freely inside the stage but cannot be
-        // hoisted out of the loop into registers (x is loop invariant), which is the whole point of keeping it in shared memory
-        int off = 0;
-#ifdef __CUDA_ARCH__
-        asm volatile("" : "+r"(off));                 // (an opaque zero offset keeps the shared address space of the pointers)
-#endif
-        double* const xp = xs + off; double* const ap = as + off;
-        const double wgt = rk.w[st];
-        const double an = rk.an[st];
-        if (st == 0) {
-#pragma unroll
-            for (int i = 0; i < 13; ++i) { ap[i * ST] = k[i]; xt[i] = fma(an, k[i], xp[i * ST]); }
-        } else if (st < 3) {
-#pragma unroll
-            for (int i = 0; i < 13; ++i) { ap[i * ST] = fma(wgt, k[i], ap[i * ST]); xt[i] = fma(an, k[i], xp[i * ST]); }
-        } else {
-#pragma unroll
-            for (int i = 0; i < 13; ++i) xp[i * ST] = fma(rk.h6, k[i] + ap[i * ST], xp[i * ST]);
-        }
-    }
 }
 
 // ---- counter-based synthetic inputs (workload definition; identical to oracle::counter_uniform) ----

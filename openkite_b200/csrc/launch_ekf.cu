@@ -1,5 +1,3 @@
-#include <cstdlib>
-
 #include "kite_launch.h"
 namespace kite {
 template <bool ARM, bool RIGID>
@@ -27,12 +25,10 @@ size_t ekf_predict_scratch_bytes() {
     return sizeof(double) * (size_t)ET_SCRATCH_PER_WARP_MAX * 8 * (size_t)sms;      // Jacobian lines of the resident warps (<= 8 per SM)
 }
 void launch_ekf_predict(const EkfArgs& a, bool rigid, bool arm, double* lines, cudaStream_t s) {
-    // the covariance moves as TMA boxes when its layout allows it (16-byte aligned base and pitch, even B);
-    // KITE_EKF_DIRECT=1 forces the direct load / store kernel (developer comparison switch)
-    static const bool direct = getenv("KITE_EKF_DIRECT") && getenv("KITE_EKF_DIRECT")[0] == '1';
+    // the covariance moves as TMA boxes when its layout allows it (16-byte aligned base and pitch, even B)
     EkfTmaArgs ta{};
     ta.e = a; ta.Jw = lines;
-    if (!direct && lines && sens_make_tensor_map(&ta.tmP, const_cast<double*>(a.P), a.B, a.ld, 169, 1) &&
+    if (lines && sens_make_tensor_map(&ta.tmP, const_cast<double*>(a.P), a.B, a.ld, 169, 1) &&
         sens_make_tensor_map(&ta.tmPn, a.Pn, a.B, a.ld, 169, 1)) {
         if (rigid) go_predict_tma<false, true>(ta, s);
         else if (arm) go_predict_tma<true, false>(ta, s);

@@ -7,9 +7,6 @@ sys.path.insert(0, ROOT)
 import numpy as np
 import torch
 import openkite_b200 as okb
-import openkite_b200.engine as _eng
-if os.environ.get("KITE_VARIANT"):
-    _eng.LIB_PATH = os.path.join(ROOT, "openkite_b200", "_variants", os.environ["KITE_VARIANT"], "libkite_b200.so")
 
 which = sys.argv[1:] or ["ekf", "colloc", "id"]
 prm = okb.load_properties(os.path.join(ROOT, "data", "umx_radian.yaml"))

@@ -1,15 +1,12 @@
 #!/usr/bin/env python
 """GPU experiment (not part of the product): time the RK4 + sensitivity step (Phi, Gamma) for one or more batch sizes.
-Usage (on the GPU box): [KITE_VARIANT=tag] [KITE_SENS_SPLIT=1] python scripts/gpu_bench_sens.py [B ...]"""
+Usage (on the GPU box): python scripts/gpu_bench_sens.py [B ...]"""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import ctypes as C
 import torch
 import openkite_b200 as okb
-import openkite_b200.engine as _eng
-if os.environ.get("KITE_VARIANT"):
-    _eng.LIB_PATH = os.path.join(ROOT, "openkite_b200", "_variants", os.environ["KITE_VARIANT"], "libkite_b200.so")
 FLOPS = 27800.0
 eng = okb.Engine(okb.load_properties(os.path.join(ROOT, "data", "umx_radian.yaml")), okb.KITE, device=0)
 peak = eng.fp64_peak(20000)
@@ -31,5 +28,5 @@ for B in [int(a) for a in sys.argv[1:]] or [262144, 1048576]:
     b.record(); torch.cuda.synchronize()
     ms = a.elapsed_time(b) / reps
     tf = FLOPS * B / (ms * 1e-3) / 1e12
-    print("%s sens B=%d: %.3f ms  %.3e units/s  %.2f TF  frac %.4f (peak %.2f)  out %.0f GB/s" % (
-        os.environ.get("KITE_VARIANT", "product"), B, ms, B / ms * 1e3, tf, tf / peak, peak, 1768.0 * B / ms / 1e6))
+    print("sens B=%d: %.3f ms  %.3e units/s  %.2f TF  frac %.4f (peak %.2f)  out %.0f GB/s" % (
+        B, ms, B / ms * 1e3, tf, tf / peak, peak, 1768.0 * B / ms / 1e6))

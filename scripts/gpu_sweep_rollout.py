@@ -6,10 +6,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import torch
 import openkite_b200 as okb
-import openkite_b200.engine as _eng
-if os.environ.get("KITE_VARIANT"):        # developer experiment: load a variant build (openkite_b200/build.py --variant)
-    _eng.LIB_PATH = os.path.join(ROOT, "openkite_b200", "_variants", os.environ["KITE_VARIANT"], "libkite_b200.so")
-    print("variant", _eng.LIB_PATH)
 
 FLOPS = 1888.0
 props = okb.load_properties(os.path.join(ROOT, "data", "umx_radian.yaml"))
