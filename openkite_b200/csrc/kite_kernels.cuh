@@ -331,6 +331,8 @@ struct SensArgs {
 // without a tether arm (127 with), so that eight warps' tiles fit one SM's shared memory.
 struct SensTab { int jx[13][13]; int ju[13][3]; int col[13][16]; };
 constexpr int SENS_SLOTS_NOARM = JAC_SLOTS_NOARM - 5, SENS_SLOTS = JAC_SLOTS - 5;
+// slots the state Jacobian spans (the EKF needs no Ju): the 99 zero-arm Jx slots come first; the tether-arm extras follow Ju
+template <bool ARM> constexpr int JX_SENS_SLOTS = ARM ? SENS_SLOTS : SENS_SLOTS_NOARM - 7;
 constexpr SensTab make_sens_tab() {
     SensTab t{};
     // value id of Qw[i][j]: +-1 = +-a0/2, +-2 = +-a1/2, +-3 = +-a2/2, 4 = s/2
@@ -690,8 +692,8 @@ __global__ void __launch_bounds__(SfCfg<ARM>::WARPS * 32, 1) k_sens_fused(const 
 // ================================================================================================
 // EKF predict (kiteEKF.cpp:75-98): xn = RK4(x,u,dt); A = I + dt Jx(x,u) at the PRE-step state; Pn = A P A^T + W.
 // One persistent kernel, every warp independent; the Jacobian never leaves the SM.
-//   phase A (lane = filter, 32 filters per group): analytic Jacobian at the pre-step state -> the warp's shared tile
-//            Jt[pass = lane / 4][slot][lane % 4], then the RK4 step -> xn.
+//   phase A (ekf_filter_step, lane = filter, 32 filters per group): the RK4 step -> xn; the Jacobian at the pre-step state
+//            -> the warp's shared tile Jt[pass = lane / 4][slot][lane % 4].
 //   phase B (8 lanes = filter, 4 filters per pass): lane l owns rows {2l, 2l+1} of P (lanes 0..6; 13 rows):
 //            Q = P A^T  (row r: q = p + dt J p), transposed through a small shared buffer, then Pn = A Q + W
 //            (column c: q + dt J q + W[:, c]).  Jacobian entries are conflict-free broadcast LDS with immediate offsets.
@@ -708,9 +710,9 @@ struct EkfArgs {
     int32_t* status;         // [ld] per-filter flags or null
 };
 template <bool ARM> struct EfCfg {
-    // state-Jacobian slots only (the EKF needs no Ju), numbered as in the sensitivity kernel (repeated +-q/2 entries share
-    // a slot): 99 without a tether arm, so that SEVEN warps' tiles and transpose buffers fit one SM
-    static constexpr int NS = ARM ? SENS_SLOTS : SENS_SLOTS_NOARM - 7;
+    // state-Jacobian slots, numbered as in the sensitivity kernel (repeated +-q/2 entries share a slot): 99 without a
+    // tether arm, so that SEVEN warps' tiles and transpose buffers fit one SM
+    static constexpr int NS = JX_SENS_SLOTS<ARM>;
     // pass stride == 4 (mod 16) doubles: the 8 four-lane groups of a phase-A store land in distinct bank octets
     static constexpr int PS = NS * 4 + ((NS * 4) % 16 == 12 ? 8 : ((NS * 4) % 16 == 0 ? 4 : (20 - (NS * 4) % 16) % 16));
     static constexpr int QR = 15;                                     // transpose buffer row stride (odd: conflict-free rows)
@@ -751,6 +753,52 @@ __device__ __forceinline__ void ekf_jx_times2(const double* __restrict__ T, cons
     }
 }
 
+// W (13 x 13 row-major) -> shared memory, one copy per CTA (the caller synchronises the block).  The kernel passes
+// threadIdx.x: read there, its range comes from the kernel's launch bounds, and with at most 169 threads the compiler
+// drops the loop's entry test.
+__device__ __forceinline__ void ekf_stage_W(double* Ws, const double* W, int tid) {
+    for (int t = tid; t < 169; t += blockDim.x) Ws[t] = __ldg(W + t);
+}
+
+// groups are claimed from a global counter: the warps of a CTA share 4 schedulers and do not all run at the same speed
+__device__ __forceinline__ long ekf_claim_group(unsigned long long* next_group, int lane) {
+    unsigned long long g = 0;
+    if (lane == 0) g = atomicAdd(next_group, 1ULL);
+    return (long)__shfl_sync(0xffffffffu, g, 0);
+}
+
+// The filter step of both predict kernels, one filter `unit` per lane: ONE evaluation of f and d f/d x at the pre-step state
+// gives the Jacobian (into `sink`) AND the first RK4 stage k1 (the reference evaluates both at the same point,
+// kiteEKF.cpp:80,93); `after_k1()` runs next, then three more RHS evaluations finish the step -> xn and the status word.
+// Ragged tail: lanes past B recompute the last filter and store nothing.
+template <bool RIGID, class Sink, class AfterK1>
+__device__ __forceinline__ void ekf_filter_step(const EkfArgs& a, long unit, Sink sink, AfterK1&& after_k1) {
+    const long ui = unit < a.B ? unit : a.B - 1;
+    double x[13], u[3], k[13], acc[13], xt[13];
+#pragma unroll
+    for (int c = 0; c < 13; ++c) x[c] = __ldcs(a.x + (long)c * a.ld + ui);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) u[c] = a.u ? __ldcs(a.u + (long)c * a.ld + ui) : 0.0;
+    const int pre = a.status ? singularity_flags<RIGID>(x) : 0;
+    model_eval<RIGID, true>(a.K, a.K.A, x, u, k, sink);
+#pragma unroll
+    for (int c = 0; c < 13; ++c) { acc[c] = k[c]; xt[c] = fma(a.rk.an[0], k[c], x[c]); }
+    after_k1();
+    NoSink ns;
+#pragma unroll 1
+    for (int st = 1; st < 4; ++st) {
+        model_eval<RIGID, false>(a.K, a.K.A, xt, u, k, ns);
+        const double wgt = a.rk.w[st], an = a.rk.an[st];
+#pragma unroll
+        for (int c = 0; c < 13; ++c) { acc[c] = fma(wgt, k[c], acc[c]); xt[c] = fma(an, k[c], x[c]); }
+    }
+    if (unit < a.B) {
+#pragma unroll
+        for (int c = 0; c < 13; ++c) { x[c] = fma(a.rk.h6, acc[c], x[c]); __stcs(a.xn + (long)c * a.ld + unit, x[c]); }
+        if (a.status) a.status[unit] = pre | (all_finite13(x) ? 0 : FLAG_NONFINITE);
+    }
+}
+
 template <bool ARM, bool RIGID>
 __global__ void __launch_bounds__(EfCfg<ARM>::WARPS * 32, 1) k_ekf_predict(const __grid_constant__ EkfArgs a) {
     using C = EfCfg<ARM>;
@@ -763,7 +811,7 @@ __global__ void __launch_bounds__(EfCfg<ARM>::WARPS * 32, 1) k_ekf_predict(const
     const int lu = lane >> 3, l = lane & 7;
     const int r0 = 2 * l, r1 = 2 * l + 1;          // rows of P (phase B, first product) = columns of Pn (second product)
     const bool v0 = r0 < 13, v1 = r1 < 13;
-    for (int t = threadIdx.x; t < 169; t += blockDim.x) Ws[t] = __ldg(a.W + t);
+    ekf_stage_W(Ws, a.W, threadIdx.x);
     __syncthreads();
     // rows r0, r1 of P for the 4 filters of a pass (registers; issued one pass ahead so the loads fly behind the FMAs)
     auto load_rows = [&](long g, int p, double (&q0)[13], double (&q1)[13]) {
@@ -776,44 +824,10 @@ __global__ void __launch_bounds__(EfCfg<ARM>::WARPS * 32, 1) k_ekf_predict(const
         }
     };
 
-    // groups are claimed from a global counter: 7 warps sit on 4 schedulers and do not all run at the same speed
-    auto claim_group = [&]() -> long {
-        unsigned long long g = 0;
-        if (lane == 0) g = atomicAdd(a.next_group, 1ULL);
-        return (long)__shfl_sync(0xffffffffu, g, 0);
-    };
-    for (long g = claim_group(); g < ngroups; g = claim_group()) {
+    for (long g = ekf_claim_group(a.next_group, lane); g < ngroups; g = ekf_claim_group(a.next_group, lane)) {
         double pn0[13], pn1[13];
         // ---------------- phase A: lane = filter ------------------------------------------------------------
-        {
-            const long unit = g * 32 + lane;
-            const long ui = unit < a.B ? unit : a.B - 1;         // ragged tail: recompute the last filter, store nothing
-            double x[13], u[3], k[13], acc[13], xt[13];
-#pragma unroll
-            for (int c = 0; c < 13; ++c) x[c] = __ldcs(a.x + (long)c * a.ld + ui);
-#pragma unroll
-            for (int c = 0; c < 3; ++c) u[c] = a.u ? __ldcs(a.u + (long)c * a.ld + ui) : 0.0;
-            const int pre = a.status ? singularity_flags<RIGID>(x) : 0;
-            {   // ONE evaluation at the pre-step state gives the Jacobian and the first RK4 stage (kiteEKF.cpp:80,93), as in the TMA kernel
-                SmemSink sink{Jt + (lane >> 2) * C::PS + (lane & 3)};
-                model_eval<RIGID, true>(a.K, a.K.A, x, u, k, sink);
-            }
-#pragma unroll
-            for (int c = 0; c < 13; ++c) { acc[c] = k[c]; xt[c] = fma(a.rk.an[0], k[c], x[c]); }
-            NoSink ns;
-#pragma unroll 1
-            for (int st = 1; st < 4; ++st) {
-                model_eval<RIGID, false>(a.K, a.K.A, xt, u, k, ns);
-                const double wgt = a.rk.w[st], an = a.rk.an[st];
-#pragma unroll
-                for (int c = 0; c < 13; ++c) { acc[c] = fma(wgt, k[c], acc[c]); xt[c] = fma(an, k[c], x[c]); }
-            }
-            if (unit < a.B) {
-#pragma unroll
-                for (int c = 0; c < 13; ++c) { x[c] = fma(a.rk.h6, acc[c], x[c]); __stcs(a.xn + (long)c * a.ld + unit, x[c]); }
-                if (a.status) a.status[unit] = pre | (all_finite13(x) ? 0 : FLAG_NONFINITE);
-            }
-        }
+        ekf_filter_step<RIGID>(a, g * 32 + lane, SmemSink{Jt + (lane >> 2) * C::PS + (lane & 3)}, [] {});
         __syncwarp();
         // (the first pass's rows are fetched here, not behind phase A: 52 more live registers across the Jacobian code spilled)
         load_rows(g, 0, pn0, pn1);
@@ -857,10 +871,9 @@ __global__ void __launch_bounds__(EfCfg<ARM>::WARPS * 32, 1) k_ekf_predict(const
 // EKF predict, round-based with TMA boxes (the product path when the covariance layout is TMA-addressable: 16-byte
 // aligned base and pitch, even B).  Same arithmetic as k_ekf_predict; what changes is how P moves and where the Jacobian
 // waits.  A warp owns groups of 32 filters:
-//   step 1 (lane = filter, 32 filters): ONE evaluation of f and d f/d x at the pre-step state gives the Jacobian AND the first
-//       RK4 stage k1 (the reference evaluates both at the same point, kiteEKF.cpp:80,93); three more RHS evaluations finish the
-//       step -> xn.  The 99 Jacobian entries of a filter go to the warp's line of an L2-resident scratch laid out
-//       [round][slot][8 filters]; the filters of round 0 also write them straight into the shared tile.  (Round 1 evaluated
+//   step 1 (ekf_filter_step, lane = filter, 32 filters): the RK4 step -> xn.  The 99 Jacobian entries of a filter go to the
+//       warp's line of an L2-resident scratch laid out [round][slot][8 filters]; the filters of round 0 also write them
+//       straight into the shared tile.  Once k1 is known, the bulk copy of round 1's tile is issued.  (Round 1 evaluated
 //       the Jacobian once per round with 4 replica lanes per filter: 30 % of the kernel's time for 3 redundant evaluations,
 //       profiles/r2a ncu source page; a 32-filter tile in shared memory would leave room for 4 warps per SM.)
 //   four rounds of 8 filters:
@@ -879,7 +892,7 @@ struct EkfTmaArgs {
     double* Jw;                       // scratch: [resident warp][4 rounds][NS slots][8 filters]
 };
 template <bool ARM> struct EtCfg {
-    static constexpr int NS = ARM ? SENS_SLOTS : SENS_SLOTS_NOARM - 7;          // state-Jacobian slots (no Ju)
+    static constexpr int NS = JX_SENS_SLOTS<ARM>;
     static constexpr int TILE_D = NS * 8;                                         // doubles per round tile [slot][8 filters]
     static constexpr unsigned TILE_BYTES = TILE_D * 8;
     static constexpr size_t BOX = (169 * 64 + 511) / 512 * 512;                   // 10816 -> 11264: both boxes see the same swizzle
@@ -892,10 +905,12 @@ template <bool ARM> struct EtCfg {
     static constexpr size_t OFF_BAR = OFF_W + sizeof(double) * 176;               // four mbarriers per warp (2 boxes, 2 tiles)
     static constexpr size_t SMEM = OFF_BAR + sizeof(unsigned long long) * 4 * WARPS;
     static constexpr long SCRATCH_PER_WARP = 4L * TILE_D;                         // doubles of L2 scratch per resident warp
+    static constexpr long SCRATCH_PER_CTA = WARPS * SCRATCH_PER_WARP;
 };
 static_assert(EtCfg<false>::SMEM <= SF_SMEM_MAX && EtCfg<true>::SMEM <= SF_SMEM_MAX, "shared memory");
 static_assert(EtCfg<false>::TILE_BYTES % 16 == 0 && EtCfg<true>::TILE_BYTES % 16 == 0, "bulk-copy granularity");
-constexpr long ET_SCRATCH_PER_WARP_MAX = EtCfg<true>::SCRATCH_PER_WARP > EtCfg<false>::SCRATCH_PER_WARP ? EtCfg<true>::SCRATCH_PER_WARP : EtCfg<false>::SCRATCH_PER_WARP;
+// doubles of Jacobian scratch per SM that ekf_predict_scratch_bytes() allocates: one CTA of either configuration
+constexpr long ET_SCRATCH_PER_CTA_MAX = EtCfg<true>::SCRATCH_PER_CTA > EtCfg<false>::SCRATCH_PER_CTA ? EtCfg<true>::SCRATCH_PER_CTA : EtCfg<false>::SCRATCH_PER_CTA;
 
 struct EkfTileSink {    // state-Jacobian slot s of this lane's filter: scratch line [round][s][8] (+ the shared tile for round 0)
     double* g;          // &Jw[lane / 8][0][lane % 8]
@@ -928,13 +943,14 @@ __global__ void __launch_bounds__(EtCfg<ARM>::WARPS * 32, 1) k_ekf_predict_tma(c
     double* const Jt = reinterpret_cast<double*>(wb + 2 * C::BOX);
     double* const Ws = reinterpret_cast<double*>(smem_raw + C::OFF_W);
     unsigned long long* const bars = reinterpret_cast<unsigned long long*>(smem_raw + C::OFF_BAR) + warp * 4;   // [box 0, box 1, tile 0, tile 1]
+    static_assert(C::WARPS * C::SCRATCH_PER_WARP <= ET_SCRATCH_PER_CTA_MAX, "the warps' scratch lines fit the host's allocation");
     double* const Jw = ta.Jw + ((long)blockIdx.x * C::WARPS + warp) * C::SCRATCH_PER_WARP;
     const long ngroups = (a.B + 31) / 32;
     const int lu = lane >> 3, l = lane & 7;
     const int r0 = l, r1 = l + 8;                  // rows of P (first product) = columns of Pn (second product)
     const bool v1 = r1 < 13;
 
-    for (int t = threadIdx.x; t < 169; t += blockDim.x) Ws[t] = __ldg(a.W + t);
+    ekf_stage_W(Ws, a.W, threadIdx.x);
     if (lane < 4) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(smem_u32(bars + lane)) : "memory");
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     __syncthreads();
@@ -958,54 +974,22 @@ __global__ void __launch_bounds__(EtCfg<ARM>::WARPS * 32, 1) k_ekf_predict_tma(c
                          :: "r"(smem_u32(Jt + (t & 1) * C::TILE_D)), "l"(Jw + (long)r * C::TILE_D), "r"(C::TILE_BYTES), "r"(bar) : "memory");
         }
     };
-    auto claim_group = [&]() -> long {
-        unsigned long long g = 0;
-        if (lane == 0) g = atomicAdd(a.next_group, 1ULL);
-        return (long)__shfl_sync(0xffffffffu, g, 0);
-    };
     unsigned t = 0;                                 // rounds done by this warp (buffer and mbarrier phase bookkeeping)
     unsigned tile_ph0 = 0, tile_ph1 = 0;            // phases of the two tile barriers (only bulk-copied rounds flip them)
-    long g = claim_group();
+    long g = ekf_claim_group(a.next_group, lane);
     if (g < ngroups) issue_load(0, g * 32);
     while (g < ngroups) {
-        const long g_next = claim_group();
-        // ---------------- step 1: lane = filter: Jacobian + k1 at the pre-step state, then the rest of the RK4 step ------
-        {
-            const long unit = g * 32 + lane;
-            const long ui = unit < a.B ? unit : a.B - 1;         // ragged tail: recompute the last filter, store nothing
-            double x[13], u[3], k[13], acc[13], xt[13];
-#pragma unroll
-            for (int c = 0; c < 13; ++c) x[c] = __ldcs(a.x + (long)c * a.ld + ui);
-#pragma unroll
-            for (int c = 0; c < 3; ++c) u[c] = a.u ? __ldcs(a.u + (long)c * a.ld + ui) : 0.0;
-            const int pre = a.status ? singularity_flags<RIGID>(x) : 0;
-            {
-                // (t is even here: a group has four rounds, so round 0 always uses tile buffer 0)
-                EkfTileSink sink{Jw + (lane >> 3) * C::TILE_D + (lane & 7), lane < 8 ? Jt + lane : nullptr};
-                model_eval<RIGID, true>(a.K, a.K.A, x, u, k, sink);
-            }
+        const long g_next = ekf_claim_group(a.next_group, lane);
+        // ---------------- step 1: lane = filter ----------------------------------------------------------------
+        // (t is even here: a group has four rounds, so round 0 always uses tile buffer 0)
+        ekf_filter_step<RIGID>(a, g * 32 + lane, EkfTileSink{Jw + (lane >> 3) * C::TILE_D + (lane & 7), lane < 8 ? Jt + lane : nullptr}, [&] {
             // the scratch lines of rounds 1..3 are read by the async proxy (bulk copies issued by lane 0)
-            // (each lane orders its own generic-proxy stores before later async-proxy reads; __syncwarp below makes them
+            // (each lane orders its own generic-proxy stores before later async-proxy reads; __syncwarp makes them
             // visible to lane 0, which issues the copy.  A full __threadfence here cost 5 % of the kernel: ERRBAR + CCTL.IVALL)
             asm volatile("fence.proxy.async;" ::: "memory");
-#pragma unroll
-            for (int c = 0; c < 13; ++c) { acc[c] = k[c]; xt[c] = fma(a.rk.an[0], k[c], x[c]); }
             __syncwarp();
             issue_tile(t + 1, 1);                  // buffer 1: last read by the previous group's round 3
-            NoSink ns;
-#pragma unroll 1
-            for (int st = 1; st < 4; ++st) {
-                model_eval<RIGID, false>(a.K, a.K.A, xt, u, k, ns);
-                const double wgt = a.rk.w[st], an = a.rk.an[st];
-#pragma unroll
-                for (int c = 0; c < 13; ++c) { acc[c] = fma(wgt, k[c], acc[c]); xt[c] = fma(an, k[c], x[c]); }
-            }
-            if (unit < a.B) {
-#pragma unroll
-                for (int c = 0; c < 13; ++c) { x[c] = fma(a.rk.h6, acc[c], x[c]); __stcs(a.xn + (long)c * a.ld + unit, x[c]); }
-                if (a.status) a.status[unit] = pre | (all_finite13(x) ? 0 : FLAG_NONFINITE);
-            }
-        }
+        });
         __syncwarp();                               // round 0's tile (written by lanes 0..7) is visible to the warp
 #pragma unroll 1
         for (int r = 0; r < 4; ++r, ++t) {

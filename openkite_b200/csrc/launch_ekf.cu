@@ -22,7 +22,7 @@ static void go_predict_tma(const EkfTmaArgs& a, cudaStream_t s) {
 size_t ekf_predict_scratch_bytes() {
     int sms = current_device_sms();        // the scratch is a per-context buffer, sized for the context's (current) device
     if (sms <= 0) sms = 256;
-    return sizeof(double) * (size_t)ET_SCRATCH_PER_WARP_MAX * 8 * (size_t)sms;      // Jacobian lines of the resident warps (<= 8 per SM)
+    return sizeof(double) * (size_t)ET_SCRATCH_PER_CTA_MAX * (size_t)sms;      // Jacobian lines of the resident warps (one CTA per SM)
 }
 void launch_ekf_predict(const EkfArgs& a, bool rigid, bool arm, double* lines, cudaStream_t s) {
     // the covariance moves as TMA boxes when its layout allows it (16-byte aligned base and pitch, even B)
