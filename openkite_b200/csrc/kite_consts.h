@@ -14,12 +14,13 @@ inline KiteConsts make_consts(const kite_params& P, int model_kind) {
     K.cqS = 0.5 * ro * P.S;
     K.b = P.b; K.c = P.c;
     K.inv_piAR = 1.0 / (pi * P.e_oswald * P.AR);
-    K.Cn0 = P.Cn0; K.Cl0 = P.Cl0;
+    K.bCn0 = P.b * P.Cn0; K.bCl0 = P.b * P.Cl0;
     K.inv_mass = 1.0 / P.mass; K.g = g;
     K.Lt = P.tether_length; K.Ks = P.Ks; K.Kd = P.Kd;
     K.arm0 = P.rx; K.arm1 = P.ry; K.arm2 = P.rz;
     K.has_arm = (P.rx != 0.0 || P.ry != 0.0 || P.rz != 0.0) ? 1 : 0;
     K.Ixx = P.Ixx; K.Iyy = P.Iyy; K.Izz = P.Izz; K.Ixz = P.Ixz;
+    K.IzmIy = P.Izz - P.Iyy; K.IymIx = P.Iyy - P.Ixx; K.IzmIx = P.Izz - P.Ixx;
     const double det = P.Ixx * P.Izz - P.Ixz * P.Ixz;     // closed-form inverse of J (SURVEY.md Q7)
     K.Ji00 = P.Izz / det; K.Ji02 = -P.Ixz / det; K.Ji11 = 1.0 / P.Iyy; K.Ji22 = P.Ixx / det;
     K.lambda = (model_kind == KITE_MODEL_RIGID_BODY) ? -10.0 : -5.0;    // kite.cpp:316 / :639

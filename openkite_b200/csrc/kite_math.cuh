@@ -110,13 +110,15 @@ static const double ANGLE_TAB[96] = KITE_ANGLE_TAB_VALUES;
 #endif
 // Angle phi in [-pi/4 - , pi/4 + ] from x = sin(phi), y = cos(phi) by table + short series instead of the degree-16 polynomial:
 //   k = rint(64 x), theta_k = asin(k / 64) from the table, d = sin(phi - theta_k) = x cos(theta_k) - y (k / 64), |d| <= 0.0112,
-//   phi = theta_k + d + d^3 (1/6 + 3/40 d^2 + 15/336 d^4)     (next term 35/1152 d^9: 7e-18 relative)
-// 11 FP64 instructions and a 9-deep dependency chain against 19 / 19; absolute error <= 3e-16 (test_lean_math_accuracy).
+//   phi = theta_k + d (1 + d^2 (1/6 + 3/40 d^2 + 15/336 d^4))     (next term 35/1152 d^9: 7e-18 relative)
+// 9 FP64 instructions and a 9-deep dependency chain against 19 / 19; absolute error <= 3e-16 (test_lean_math_accuracy).
+// k / 64 comes straight out of the rounding constant (t / 64 - magic / 64 is exact), and the series ends in one FMA onto
+// theta_k, so no instruction reads three fresh vector registers.
 // The product kernels use this form everywhere: config 2 81.38 -> 80.10 ms against the polynomial (profiles/r2r_sweep.log).
 __device__ __forceinline__ double asin_red(double x, double y) {
     const double magic = 6755399441055744.0;              // 1.5 * 2^52: the low word of x * 64 + magic is rint(64 x)
     const double t = fma(x, 64.0, magic);
-    const double kf = t - magic;
+    const double kf = fma(t, 0.015625, -magic * 0.015625);  // k / 64, exact
 #ifdef __CUDA_ARCH__
     int k = __double2loint(t);
     k = k < 0 ? -k : k;
@@ -128,11 +130,12 @@ __device__ __forceinline__ double asin_red(double x, double y) {
     k = k < 0 ? -k : k;
     const double ck = ANGLE_TAB[2 * k], thk = ANGLE_TAB[2 * k + 1];
 #endif
-    const double d = fma(y * kf, -0.015625, x * ck);
+    const double d = fma(-y, kf, x * ck);
     const double u = d * d;
     double p = fma(4.46428571428571425e-02, u, 7.49999999999999972e-02);
     p = fma(p, u, 1.66666666666666657e-01);
-    return copysign(thk, kf) + fma(d * u, p, d);
+    p = fma(p, u, 1.0);
+    return fma(d, p, copysign(thk, kf));
 }
 // Angle in [-pi/2, pi/2] from its sine s and cosine c >= 0 (s^2 + c^2 = 1), branch free over the whole range:
 //   |s| <= 1/sqrt2 : asin(s)            |s| > 1/sqrt2 : sign(s) (pi/2 - asin(c)),  c < 1/sqrt2
@@ -163,26 +166,29 @@ static __device__ const double EXP2_TAB[32] = KITE_EXP2_TAB_VALUES;
 static const double EXP2_TAB[32] = KITE_EXP2_TAB_VALUES;
 #endif
 
-// logistic(x) = 1 / (1 + exp(-x)); argument clamped to +-700 (result 0 / 1 to within 1e-304 beyond).
+// logistic(4 e) = 1 / (1 + exp(-4 e)), the tether's smoothed step; argument clamped to |4 e| <= 700 (result 0 / 1 to within
+// 1e-304 beyond).  exp(a) at a = -4 e is evaluated on the reduced argument r' = r / (-4): every literal below is the one of
+// the plain exp(a) form times a power of two ((-4)^k for the k-th polynomial coefficient, -1/4 for the reduction constants,
+// -4 for the rounding product), so each rounding lands on the same scaled value and the result is bitwise that of exp(a)
+// with a = -4 e, without the FP64 instruction that forms a.
 template <bool TAB>
-__device__ __forceinline__ double fast_logistic(double x) {
-    double a = -x;
-    a = fmin(fmax(a, -700.0), 700.0);
+__device__ __forceinline__ double fast_logistic4(double e) {
+    e = fmax(fmin(e, 175.0), -175.0);
     if constexpr (TAB)
     // exp(a) = 2^m * 2^(j/32) * exp(r): n = rint(a * 32 / ln2) = 32 m + j, r = a - n ln2/32 (Cody-Waite), |r| <= ln2/64 = 0.0108,
     // exp(r) by a degree-6 Taylor polynomial (r^7/5040 = 3.5e-18): 12 FP64 instructions against 17 with the degree-11 one.
     {
         const double magic = 6755399441055744.0;
-        const double tn = fma(a, 4.61662413084468283e+01, magic);
+        const double tn = fma(e, -4.0 * 4.61662413084468283e+01, magic);
         const double nf = tn - magic;
-        double r = fma(nf, -2.16608493865351193e-02, a);
-        r = fma(nf, -5.96317165397058656e-12, r);
-        double p = 1.38888888888888894e-03;
-        p = fma(p, r, 8.33333333333333322e-03);
-        p = fma(p, r, 4.16666666666666644e-02);
-        p = fma(p, r, 1.66666666666666657e-01);
-        p = fma(p, r, 5.00000000000000000e-01);
-        p = fma(p, r, 1.00000000000000000e+00);
+        double r = fma(nf, 0.25 * 2.16608493865351193e-02, e);
+        r = fma(nf, 0.25 * 5.96317165397058656e-12, r);
+        double p = 4096.0 * 1.38888888888888894e-03;
+        p = fma(p, r, -1024.0 * 8.33333333333333322e-03);
+        p = fma(p, r, 256.0 * 4.16666666666666644e-02);
+        p = fma(p, r, -64.0 * 1.66666666666666657e-01);
+        p = fma(p, r, 16.0 * 5.00000000000000000e-01);
+        p = fma(p, r, -4.0 * 1.00000000000000000e+00);
         p = fma(p, r, 1.00000000000000000e+00);
         int64_t bits;
         memcpy(&bits, &tn, sizeof bits);
@@ -200,22 +206,22 @@ __device__ __forceinline__ double fast_logistic(double x) {
     }
     // n = rint(a * log2(e)) by the 1.5 * 2^52 trick; r = a - n ln2 (Cody-Waite, hi part has 32 trailing zero bits)
     const double magic = 6755399441055744.0;
-    const double tn = fma(a, 1.44269504088896339e+00, magic);
+    const double tn = fma(e, -4.0 * 1.44269504088896339e+00, magic);
     const double nf = tn - magic;
-    double r = fma(nf, -6.93146705627441406e-01, a);
-    r = fma(nf, -4.74932503903167256e-07, r);
+    double r = fma(nf, 0.25 * 6.93146705627441406e-01, e);
+    r = fma(nf, 0.25 * 4.74932503903167256e-07, r);
     // exp(r), |r| <= ln2/2, degree 11 (scripts/fit_math_polys.py)
-    double p = 2.51100492048186583e-08;
-    p = fma(p, r, 2.76326547225277896e-07);
-    p = fma(p, r, 2.75572408872298695e-06);
-    p = fma(p, r, 2.48014854415613131e-05);
-    p = fma(p, r, 1.98412698900764028e-04);
-    p = fma(p, r, 1.38888889523528631e-03);
-    p = fma(p, r, 8.33333333331958900e-03);
-    p = fma(p, r, 4.16666666664879531e-02);
-    p = fma(p, r, 1.66666666666666796e-01);
-    p = fma(p, r, 5.00000000000001887e-01);
-    p = fma(p, r, 1.00000000000000000e+00);
+    double p = -4194304.0 * 2.51100492048186583e-08;
+    p = fma(p, r, 1048576.0 * 2.76326547225277896e-07);
+    p = fma(p, r, -262144.0 * 2.75572408872298695e-06);
+    p = fma(p, r, 65536.0 * 2.48014854415613131e-05);
+    p = fma(p, r, -16384.0 * 1.98412698900764028e-04);
+    p = fma(p, r, 4096.0 * 1.38888889523528631e-03);
+    p = fma(p, r, -1024.0 * 8.33333333331958900e-03);
+    p = fma(p, r, 256.0 * 4.16666666664879531e-02);
+    p = fma(p, r, -64.0 * 1.66666666666666796e-01);
+    p = fma(p, r, 16.0 * 5.00000000000001887e-01);
+    p = fma(p, r, -4.0 * 1.00000000000000000e+00);
     p = fma(p, r, 1.00000000000000000e+00);
     // scale by 2^n: n is in the low word of tn (|n| <= 1010, so the biased exponent stays normal)
     int64_t bits;
@@ -224,8 +230,13 @@ __device__ __forceinline__ double fast_logistic(double x) {
     const int64_t sb = (n + 1023) << 52;
     double scale;
     memcpy(&scale, &sb, sizeof scale);
-    const double ex = p * scale;                  // exp(-x)
+    const double ex = p * scale;                  // exp(-4 e)
     return fast_rcp(1.0 + ex);
+}
+// logistic(x) = 1 / (1 + exp(-x)): x / 4 is exact, so this is bitwise the logistic of x.
+template <bool TAB>
+__device__ __forceinline__ double fast_logistic(double x) {
+    return fast_logistic4<TAB>(0.25 * x);
 }
 
 }  // namespace kite

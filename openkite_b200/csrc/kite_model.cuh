@@ -23,12 +23,15 @@ namespace kite {
 
 // Derived aerodynamic coefficients (from the 21 raw coefficients, kite.cpp:571-572 order).
 struct AeroCoef {
-    double CL0, CLa, CD0, CYb, Cm0, Cma, Cnb, Clb;
+    double CL0, CLa, CD0, CYb;
+    double cCm0, cCma;       // c*{Cm0,Cma}: the pitch moment is (c Cm) q S (kite.cpp:278), so the chord is folded in here
+    double bCnb, bClb;       // b*{Cnb,Clb}: likewise the span for the yaw / roll moments (kite.cpp:274,282)
     double kLq;              // 0.25*CLq*c*S*ro          (kite.cpp:210)
     double kmq;              // Cmq*0.25*S*c^2*ro        (kite.cpp:279)
     double kYr, kYp;         // 0.25*b*ro*S*{CYr,CYp}    (kite.cpp:213)
     double knr, klr, klp, knp;  // 0.25*ro*b^2*S*{Cnr,Clr,Clp,Cnp}  (kite.cpp:275,283)
-    double CLde, CYdr, Cmde, Cndr, Cldr;
+    double CLde, CYdr;
+    double cCmde, bCndr, bCldr;  // c*Cmde, b*Cndr, b*Cldr
 };
 
 // Which coefficient types select the table-driven exponential (kite_eval_c): volatile AeroCoef (identification sweeps, per-
@@ -44,11 +47,12 @@ struct KiteConsts {
     double cqS;              // 0.5*ro*S  -> qS = cqS*V^2 (dynamic pressure times wing area)
     double b, c;
     double inv_piAR;         // 1/(pi*e_o*AR)
-    double Cn0, Cl0;
+    double bCn0, bCl0;       // b*Cn0, b*Cl0
     double inv_mass, g;
     double Lt, Ks, Kd;
     double arm0, arm1, arm2; // tether attachment arm (rx,ry,rz)
     double Ixx, Iyy, Izz, Ixz, Ji00, Ji02, Ji11, Ji22;
+    double IzmIy, IymIx, IzmIx;  // Izz-Iyy, Iyy-Ixx, Izz-Ixx: w x (J w) in factored form
     double lambda;           // quaternion-norm stabiliser gain: -5 kite, -10 rigid body
     double sLq, smq, sY, sb2;  // factors that turn raw CLq, Cmq, CY*, C{l,n}* into AeroCoef entries
     int has_arm;
@@ -56,7 +60,8 @@ struct KiteConsts {
 };
 
 __host__ __device__ inline void derive_coef(const KiteConsts& K, const double p[21], AeroCoef& A) {
-    A.CL0 = p[0]; A.CLa = p[1]; A.CD0 = p[2]; A.CYb = p[3]; A.Cm0 = p[4]; A.Cma = p[5]; A.Cnb = p[6]; A.Clb = p[7];
+    A.CL0 = p[0]; A.CLa = p[1]; A.CD0 = p[2]; A.CYb = p[3];
+    A.cCm0 = K.c * p[4]; A.cCma = K.c * p[5]; A.bCnb = K.b * p[6]; A.bClb = K.b * p[7];
     A.kLq = K.sLq * p[8];
     A.kmq = K.smq * p[9];
     A.kYr = K.sY * p[10];
@@ -65,7 +70,7 @@ __host__ __device__ inline void derive_coef(const KiteConsts& K, const double p[
     A.kYp = K.sY * p[13];
     A.klp = K.sb2 * p[14];
     A.knp = K.sb2 * p[15];
-    A.CLde = p[16]; A.CYdr = p[17]; A.Cmde = p[18]; A.Cndr = p[19]; A.Cldr = p[20];
+    A.CLde = p[16]; A.CYdr = p[17]; A.cCmde = K.c * p[18]; A.bCndr = K.b * p[19]; A.bCldr = K.b * p[20];
 }
 
 // ---- small helpers ---------------------------------------------------------------------
@@ -128,21 +133,21 @@ struct NoSink {
 // Everything the right-hand side needs from the control u = [T dE dR]: the five coefficient sums that are affine in dE / dR.
 // RK4 holds u for all four stages (kitemath.cpp:36-51), so the integrators evaluate these once per step, not per stage.
 struct CtrlTerms {
-    double T;        // thrust
+    double Tm;       // thrust / mass
     double cydr;     // CYdr dR                 (side force,  kite.cpp:212)
-    double cl0;      // Cl0 + Cldr dR           (roll moment, kite.cpp:274)
-    double cm0;      // Cm0 + Cmde dE           (pitch moment, kite.cpp:278)
-    double cn0;      // Cn0 + Cndr dR           (yaw moment,  kite.cpp:282)
+    double cl0;      // b (Cl0 + Cldr dR)       (roll moment, kite.cpp:274)
+    double cm0;      // c (Cm0 + Cmde dE)       (pitch moment, kite.cpp:278)
+    double cn0;      // b (Cn0 + Cndr dR)       (yaw moment,  kite.cpp:282)
     double nzde;     // -CLde dE                (elevator force / (q S), kite.cpp:228)
 };
 template <class AC>
 __device__ __forceinline__ CtrlTerms ctrl_terms(const KiteConsts& K, const AC& A, const double (&u)[3]) {
     CtrlTerms c;
-    c.T = u[0];
+    c.Tm = u[0] * K.inv_mass;
     c.cydr = A.CYdr * u[2];
-    c.cl0 = fma(A.Cldr, u[2], K.Cl0);
-    c.cm0 = fma(A.Cmde, u[1], A.Cm0);
-    c.cn0 = fma(A.Cndr, u[2], K.Cn0);
+    c.cl0 = fma(A.bCldr, u[2], K.bCl0);
+    c.cm0 = fma(A.cCmde, u[1], A.cCm0);
+    c.cn0 = fma(A.bCndr, u[2], K.bCn0);
     c.nzde = -A.CLde * u[1];
     return c;
 }
@@ -179,15 +184,16 @@ __device__ __forceinline__ void kite_eval_c(const KiteConsts& K, const AC& A, co
     const double ss = asin_sc<true>(sb, cb);
     const double aoa = atan2_sc<true>(sa, ca);
     const double qS = K.cqS * V2;
+    // rate damping terms are linear in V w: the airspeed scales the rates once, not each coefficient sum
+    const double Vw0 = V * w[0], Vw1 = V * w[1], Vw2 = V * w[2];
 
     // ---- aerodynamic force in the wind frame, rotated to body ---------------------------
     const double CL = fma(A.CLa, aoa, A.CL0);
     const double CD = fma(CL * CL, K.inv_piAR, A.CD0);
-    const double LIFT = fma(CL, qS, A.kLq * V * w[1]);
+    const double LIFT = fma(CL, qS, A.kLq * Vw1);
     const double DRAG = CD * qS;
     const double cy = fma(A.CYb, ss, uc.cydr);
-    const double kYw = fma(A.kYr, w[2], A.kYp * w[0]);
-    const double SF = fma(cy, qS, kYw * V);
+    const double SF = fma(cy, qS, fma(A.kYr, Vw2, A.kYp * Vw0));
     const double Zde = uc.nzde * qS;
     const double X1 = fma(sa, LIFT, -ca * DRAG);
     const double Z1 = -fma(sa, DRAG, ca * LIFT);
@@ -217,7 +223,7 @@ __device__ __forceinline__ void kite_eval_c(const KiteConsts& K, const AC& A, co
     const double d = d2 * id;
     const double n[3] = {r[0] * id, r[1] * id, r[2] * id};
     const double e = d - K.Lt;
-    const double H = fast_logistic<TAB>(4.0 * e);                   // K/(1+exp(-4x)), kitemath.cpp:31-34
+    const double H = fast_logistic4<TAB>(e);                        // K/(1+exp(-4x)), kitemath.cpp:31-34
     const double nv = fma(n[0], vi[0], fma(n[1], vi[1], n[2] * vi[2]));
     const double tens = fma(K.Ks, e, K.Kd * nv);
     const double tau = tens * H;
@@ -228,33 +234,32 @@ __device__ __forceinline__ void kite_eval_c(const KiteConsts& K, const AC& A, co
     for (int i = 0; i < 3; ++i) m[i] = fma(M[1][i], n[1], m[i]);
 #pragma unroll
     for (int i = 0; i < 3; ++i) m[i] = fma(M[0][i], n[0], m[i]);
-    const double Rb[3] = {-tau * m[0], -tau * m[1], -tau * m[2]};     // only consumed by the tether-arm moment and the Jacobian
 
-    // ---- v_dot = (Faero + T e1 + R_b)/m + g M^T e3 - w x v ---------------------------------
+    // ---- v_dot = (Faero + T e1 + R_b)/m + g M^T e3 - w x v,  R_b = -tau m ------------------
     const double tm = -tau * K.inv_mass;                              // R_b / mass = tm * m
-    f[0] = fma(tm, m[0], fma(Fx + uc.T, K.inv_mass, fma(K.g, M[2][0], fma(w[2], v[1], -w[1] * v[2]))));
+    f[0] = fma(tm, m[0], fma(Fx, K.inv_mass, fma(K.g, M[2][0], fma(w[2], v[1], fma(-w[1], v[2], uc.Tm)))));
     f[1] = fma(tm, m[1], fma(Fy, K.inv_mass, fma(K.g, M[2][1], fma(w[0], v[2], -w[2] * v[0]))));
     f[2] = fma(tm, m[2], fma(Fz, K.inv_mass, fma(K.g, M[2][2], fma(w[1], v[0], -w[0] * v[1]))));
 
-    // ---- moments ---------------------------------------------------------------------------
-    const double qSb = qS * K.b, qSc = qS * K.c;
-    const double cl = fma(A.Clb, ss, uc.cl0);
-    const double cm = fma(A.Cma, aoa, uc.cm0);
-    const double cn = fma(A.Cnb, ss, uc.cn0);
-    const double klw = fma(A.klr, w[2], A.klp * w[0]);
-    const double knw = fma(A.knp, w[0], A.knr * w[2]);
-    const double Lm = fma(cl, qSb, klw * V);
-    const double Mm = fma(cm, qSc, A.kmq * w[1] * V);
-    const double Nm = fma(cn, qSb, knw * V);
+    // ---- moments (b and c are folded into the coefficient sums: cl = b Cl, cm = c Cm, cn = b Cn) ----
+    const double cl = fma(A.bClb, ss, uc.cl0);
+    const double cm = fma(A.cCma, aoa, uc.cm0);
+    const double cn = fma(A.bCnb, ss, uc.cn0);
+    const double Lm = fma(cl, qS, fma(A.klr, Vw2, A.klp * Vw0));
+    const double Mm = fma(cm, qS, A.kmq * Vw1);
+    const double Nm = fma(cn, qS, fma(A.knp, Vw0, A.knr * Vw2));
     const double Max = fma(ca, Lm, -sa * Nm);
     const double Maz = fma(sa, Lm, ca * Nm);
-    const double Jw0 = fma(K.Ixx, w[0], K.Ixz * w[2]);
-    const double Jw1 = K.Iyy * w[1];
-    const double Jw2 = fma(K.Ixz, w[0], K.Izz * w[2]);
-    double rh0 = Max - (w[1] * Jw2 - w[2] * Jw1);
-    double rh1 = Mm - (w[2] * Jw0 - w[0] * Jw2);
-    double rh2 = Maz - (w[0] * Jw1 - w[1] * Jw0);
+    // rh = M_aero - w x (J w) with J = [Ixx 0 Ixz; 0 Iyy 0; Ixz 0 Izz], factored:
+    //   (w x J w)_0 = w1 (Ixz w0 + (Izz-Iyy) w2),  (w x J w)_2 = w1 ((Iyy-Ixx) w0 - Ixz w2),
+    //   (w x J w)_1 = (Ixx-Izz) w0 w2 + Ixz (w2^2 - w0^2)
+    const double G0 = fma(K.Ixz, w[0], K.IzmIy * w[2]);
+    const double G2 = fma(K.IymIx, w[0], -K.Ixz * w[2]);
+    double rh0 = fma(-w[1], G0, Max);
+    double rh1 = fma(K.IzmIx, w[0] * w[2], fma(K.Ixz, fma(w[0], w[0], -w[2] * w[2]), Mm));
+    double rh2 = fma(-w[1], G2, Maz);
     if (K.has_arm) {
+        const double Rb[3] = {-tau * m[0], -tau * m[1], -tau * m[2]};
         rh0 += K.arm1 * Rb[2] - K.arm2 * Rb[1];
         rh1 += K.arm2 * Rb[0] - K.arm0 * Rb[2];
         rh2 += K.arm0 * Rb[1] - K.arm1 * Rb[0];
@@ -265,7 +270,8 @@ __device__ __forceinline__ void kite_eval_c(const KiteConsts& K, const AC& A, co
 
     // ---- kinematics --------------------------------------------------------------------------
     f[6] = vi[0]; f[7] = vi[1]; f[8] = vi[2];
-    const double mu = (0.5 * K.lambda) * (nq - 1.0);
+    const double hl = 0.5 * K.lambda;
+    const double mu = fma(nq, hl, -hl);                                // (lambda / 2) (|q|^2 - 1)
     const double hw[3] = {0.5 * w[0], 0.5 * w[1], 0.5 * w[2]};         // q_dot = q (x) [0, w/2] + mu q
     // (sweeps over hw[2], hw[1], hw[0], mu: each shares its second operand across the four rows)
     f[9] = -a[2] * hw[2];                 f[10] = a[1] * hw[2];                 f[11] = -a[0] * hw[2];                f[12] = s * hw[2];
@@ -274,6 +280,13 @@ __device__ __forceinline__ void kite_eval_c(const KiteConsts& K, const AC& A, co
     f[9] = fma(s, mu, f[9]);              f[10] = fma(a[0], mu, f[10]);         f[11] = fma(a[1], mu, f[11]);         f[12] = fma(a[2], mu, f[12]);
 
     if constexpr (JAC) {
+        const double Rb[3] = {-tau * m[0], -tau * m[1], -tau * m[2]};
+        const double kYw = fma(A.kYr, w[2], A.kYp * w[0]);
+        const double klw = fma(A.klr, w[2], A.klp * w[0]);
+        const double knw = fma(A.knp, w[0], A.knr * w[2]);
+        const double Jw0 = fma(K.Ixx, w[0], K.Ixz * w[2]);
+        const double Jw1 = K.Iyy * w[1];
+        const double Jw2 = fma(K.Ixz, w[0], K.Izz * w[2]);
         // =========================== gradients w.r.t. v of the aero scalars =======================
         const double dV[3] = {v[0] * rV, v[1] * rV, v[2] * rV};
         const double icb = rcb;
@@ -300,9 +313,9 @@ __device__ __forceinline__ void kite_eval_c(const KiteConsts& K, const AC& A, co
             dFx[j] = fma(dcb, X1, fma(cb, dX1, -fma(dsa, Zde, sa * dZde)));
             dFy[j] = fma(dsb, X1, fma(sb, dX1, dSF));
             dFz[j] = dZ1 + fma(dca, Zde, ca * dZde);
-            const double dLm = fma(A.Clb * qSb, dss[j], fma(cl * K.b, dqS[j], klw * dV[j]));
-            const double dMm = fma(A.Cma * qSc, daoa[j], fma(cm * K.c, dqS[j], A.kmq * w[1] * dV[j]));
-            const double dNm = fma(A.Cnb * qSb, dss[j], fma(cn * K.b, dqS[j], knw * dV[j]));
+            const double dLm = fma(A.bClb * qS, dss[j], fma(cl, dqS[j], klw * dV[j]));
+            const double dMm = fma(A.cCma * qS, daoa[j], fma(cm, dqS[j], A.kmq * w[1] * dV[j]));
+            const double dNm = fma(A.bCnb * qS, dss[j], fma(cn, dqS[j], knw * dV[j]));
             dMax[j] = fma(-Maz, daoa[j], fma(ca, dLm, -sa * dNm));
             dMy[j] = dMm;
             dMaz[j] = fma(Max, daoa[j], fma(sa, dLm, ca * dNm));
@@ -442,8 +455,8 @@ __device__ __forceinline__ void kite_eval_c(const KiteConsts& K, const AC& A, co
         }
         // d/du
         {
-            const double MdE = A.Cmde * qSc;
-            const double LdR = A.Cldr * qSb, NdR = A.Cndr * qSb;
+            const double MdE = A.cCmde * qS;
+            const double LdR = A.bCldr * qS, NdR = A.bCndr * qS;
             const double r0 = fma(ca, LdR, -sa * NdR), r2 = fma(sa, LdR, ca * NdR);
             sink.ju(4, 1, K.Ji11 * MdE);
             sink.ju(3, 2, fma(K.Ji00, r0, K.Ji02 * r2));
@@ -498,7 +511,8 @@ __device__ __forceinline__ void rigid_eval(const KiteConsts& K, const double (&x
     for (int i = 0; i < 6; ++i) f[i] = 0.0;
 #pragma unroll
     for (int i = 0; i < 3; ++i) f[6 + i] = fma(M[i][0], v[0], fma(M[i][1], v[1], M[i][2] * v[2]));
-    const double mu = (0.5 * K.lambda) * (nq - 1.0);
+    const double hl = 0.5 * K.lambda;
+    const double mu = fma(nq, hl, -hl);                                // (lambda / 2) (|q|^2 - 1)
     const double hw[3] = {0.5 * w[0], 0.5 * w[1], 0.5 * w[2]};         // q_dot = q (x) [0, w/2] + mu q
     f[9] = fma(mu, s, -fma(a[0], hw[0], fma(a[1], hw[1], a[2] * hw[2])));
     f[10] = fma(mu, a[0], fma(s, hw[0], fma(a[1], hw[2], -a[2] * hw[1])));

@@ -3,12 +3,15 @@
 registers / stack / spill bytes of every kernel (`-Xptxas -v`), and per kernel the SASS instruction histogram, the TMA /
 mbarrier mnemonics that prove the bulk-tensor paths, and -- for the rollout kernels -- the FP64 instructions of the stage
 loop by the number of distinct vector-register operands not served by the reuse cache (the operand-delivery cost model of
-DESIGN.md section 7: cycles = sum of max(2, operands)).      python scripts/sass_report.py <tag>"""
+DESIGN.md section 7: cycles = sum of max(2, operands)).  profiles/<tag>_stage_loop.txt lists every FP64 instruction of those
+stage loops with its uncached-operand count and the source line it comes from (nvdisasm line table of the -lineinfo build).
+    python scripts/sass_report.py <tag>"""
 import collections
 import os
 import re
 import subprocess
 import sys
+import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -26,9 +29,32 @@ def parse(sass):
     return rows
 
 
-def operand_model(rows, lo, hi):
+def source_lines(obj, fn):
+    """{address: 'file:line'} of kernel `fn` in `obj`, from nvdisasm's line table."""
+    out, src, inside = {}, "?", False
+    with tempfile.TemporaryDirectory() as d:
+        subprocess.run(["cuobjdump", "-xelf", "all", os.path.abspath(obj)], cwd=d, capture_output=True)
+        for cub in sorted(f for f in os.listdir(d) if f.endswith(".cubin")):
+            txt = subprocess.run(["nvdisasm", "-g", "-c", os.path.join(d, cub)], capture_output=True, text=True).stdout
+            for ln in txt.splitlines():
+                if ln.startswith("//----"):
+                    inside = fn in ln
+                    continue
+                if not inside:
+                    continue
+                m = re.match(r'\s*//## File "([^"]+)", line (\d+)', ln)
+                if m:
+                    src = "%s:%s" % (os.path.basename(m.group(1)), m.group(2))
+                    continue
+                m = re.match(r"\s+/\*([0-9a-f]{4,})\*/", ln)
+                if m:
+                    out[int(m.group(1), 16)] = src
+    return out
+
+
+def operand_model(rows, lo, hi, listing=None):
     prev, stats, cyc = {}, collections.Counter(), 0
-    for a, op, _, ops in rows:
+    for a, op, full, ops in rows:
         if not (lo <= a <= hi):
             continue
         srcs = ops[1:] if op != "DSETP" else ops[2:]
@@ -46,6 +72,8 @@ def operand_model(rows, lo, hi):
                         cur[i] = reg
             stats[nv] += 1
             cyc += max(2, nv)
+            if listing is not None:
+                listing.append((a, nv, full, ", ".join(ops)))
         else:
             for i, o in enumerate(srcs):
                 mm = re.match(r"[-|~]*(R\d+)\.reuse", o)
@@ -64,6 +92,9 @@ def main():
         for name, regs, stack, sst, sld in kb.resource_report():
             dem = subprocess.run(["c++filt", name], capture_output=True, text=True).stdout.strip()
             fh.write("%-88s regs=%3d stack=%4d spill_st=%4d spill_ld=%4d\n" % (dem[:88], regs, stack, sst, sld))
+    loop_fh = open(os.path.join(out, "%s_stage_loop.txt" % tag), "w")
+    loop_fh.write("FP64 instructions of the rollout stage loops: address, vector-register operands not served by the reuse cache, "
+                  "instruction, source line\n")
     with open(os.path.join(out, "%s_sass_histogram.txt" % tag), "w") as fh:
         fh.write("cuobjdump -sass of openkite_b200/_obj/*.o (sm_100a): instruction histograms of the product kernels\n")
         for unit, pat in (("launch_rollout_a", "k_rk4_rolloutILi1ELb0ELb0"), ("launch_rollout_b", "k_rk4_rolloutILi2ELb0ELb1"),
@@ -95,12 +126,20 @@ def main():
             if "rollout" in pat and loops:
                 lo, hi = loops[0]
                 body = collections.Counter(op for a, op, _, _ in rows if lo <= a <= hi)
-                stats, cyc = operand_model(rows, lo, hi)
+                listing = []
+                stats, cyc = operand_model(rows, lo, hi, listing)
                 n = sum(stats.values())
+                src = source_lines(obj, fn[0])
+                loop_fh.write("\n== %s  stage loop 0x%x-0x%x\n" % (dem, lo, hi))
+                by_line = collections.Counter(src.get(a, "?") for a, nv, _, _ in listing if nv >= 3)
+                loop_fh.write("three-operand instructions by source line: %s\n" % ", ".join("%s %d" % kv for kv in sorted(by_line.items())))
+                for a, nv, full, ops in listing:
+                    loop_fh.write("%04x %s %-7s %-44s %s\n" % (a, "*3" if nv >= 3 else " %d" % nv, full, ops, src.get(a, "?")))
                 fh.write("stage loop 0x%x-0x%x: %d instructions, %d on the FP64 pipe (%s)\n" %
                          (lo, hi, sum(body.values()), n, ", ".join("%s %d" % (k, body[k]) for k in FP64)))
                 fh.write("  FP64 instructions by uncached vector-register operands: %s -> %d cycles per stage at max(2, operands) (%.2f per instruction)\n" %
                          (dict(sorted(stats.items())), cyc, cyc / max(n, 1)))
+    loop_fh.close()
     print(open(os.path.join(out, "%s_sass_histogram.txt" % tag)).read())
 
 
