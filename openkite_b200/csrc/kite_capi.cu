@@ -407,7 +407,7 @@ static int sens_impl(kite_ctx* ctx, long B, long ld, long N, double h, const dou
     if (ctx->counters.reserve(64)) return fail(ctx, KITE_ERR_CUDA, "cudaMalloc failed");
     CK(cudaMemsetAsync(ctx->counters.ptr, 0, 8, ctx->stream));
     SensArgs a{};
-    a.K = ctx->K; a.B = B; a.ld = ld; a.N = N; a.h = h; a.x = x; a.u = u; a.xn = xn; a.Phi = Phi; a.Gamma = Gamma;
+    a.K = ctx->K; a.B = B; a.ld = ld; a.N = N; a.rk = make_rk_tab(h); a.x = x; a.u = u; a.xn = xn; a.Phi = Phi; a.Gamma = Gamma;
     a.Sw = (double*)work; a.next_group = (unsigned long long*)ctx->counters.ptr;
     a.done = (int*)((char*)work + sens_state_bytes(B));
     if (N > 1) CK(cudaMemsetAsync(a.done, 0, sizeof(int) * (size_t)((B + 31) / 32), ctx->stream));

@@ -315,7 +315,7 @@ struct SensArgs {
     KiteConsts K;
     long B, ld;
     long N;                           // steps of the multiple-shooting rollout (1: a single step)
-    double h;
+    RkTab rk;                         // RK4 tableau for h (host-computed)
     const double* x; const double* u; // x [13][ld] (state before step 0), u [N][3][ld]
     double* xn; double* Phi; double* Gamma;   // xn [N][13][ld] (state after each step), Phi [N][169][ld], Gamma [N][39][ld]
     double* Sw;     // scratch: [resident warp][4 stages][16 = x(13) | u(3)][32 units]
@@ -425,6 +425,45 @@ struct StageSink {      // the warp's tile: slot s of this lane's (unit, stage) 
     __device__ __forceinline__ void aero(double, double, double) const {}
 };
 
+// y = J v for two vectors at once: J = [Jx | Ju] (NC = 16 input columns) or Jx (NC = 13) in compact slots, read from the
+// shared tile column of one unit (tile rows [slot][STRIDE units]).
+// The control columns 13..15 update y1 only.  The one caller with NC = 16 (phase B of k_sens_fused) passes the control
+// part of its seed there, which is 0 in v0 (the lane's first tangent column c0 < 8 is a column of Phi) and e_(c1 - 13) in
+// v1.  The zero products must be skipped, not just saved: fma(jv, 0, y) is not bitwise y (-0 + 0 gives +0, and an
+// infinite or NaN entry gives NaN).
+// Column-major traversal: the (up to 13) entries J[i][j] of input row j update 26 independent chains, so consecutive DFMAs
+// never depend on each other.  Operand order matters: a DFMA with three distinct vector-register operands issues every 3
+// cycles, with two every 2 (profiles/r2j_dfma_operands.log).  The two FMAs of an entry share jv; alternating which vector
+// goes first makes the first FMA of the NEXT entry share v[.][j] with the one before it, so that every FMA finds one
+// operand in the reuse cache: ... (v0, jv1) (v1, jv1) (v1, jv2) (v0, jv2) (v0, jv3) ...
+template <bool ARM, bool RIGID, int STRIDE, int NC>
+__device__ __forceinline__ void jac_times2(const double* __restrict__ T, const double (&v0)[NC], const double (&v1)[NC],
+                                           double (&y0)[13], double (&y1)[13]) {
+    static_assert(NC == 13 || NC == 16, "Jx or [Jx | Ju]");
+#pragma unroll
+    for (int i = 0; i < 13; ++i) { y0[i] = 0.0; y1[i] = 0.0; }
+    int flip = 0;
+#pragma unroll
+    for (int j = 0; j < NC; ++j) {
+#pragma unroll
+        for (int i = (RIGID ? 6 : 0); i < 13; ++i) {
+            if ((j < 13) ? jx_nz(i, j, ARM) : (!RIGID && ju_nz(i, j - 13))) {
+                const double jv = T[SENS_TAB.col[i][j] * STRIDE];     // broadcast LDS.64, immediate offset
+                if (j >= 13) {
+                    y1[i] = fma(jv, v1[j], y1[i]);
+                } else if (flip) {
+                    y1[i] = fma(jv, v1[j], y1[i]);
+                    y0[i] = fma(jv, v0[j], y0[i]);
+                } else {
+                    y0[i] = fma(jv, v0[j], y0[i]);
+                    y1[i] = fma(jv, v1[j], y1[i]);
+                }
+                flip ^= 1;
+            }
+        }
+    }
+}
+
 template <bool ARM, bool RIGID, bool TMA_OUT>
 __global__ void __launch_bounds__(SfCfg<ARM>::WARPS * 32, 1) k_sens_fused(const __grid_constant__ SensArgs a) {
     using C = SfCfg<ARM>;
@@ -471,7 +510,7 @@ __global__ void __launch_bounds__(SfCfg<ARM>::WARPS * 32, 1) k_sens_fused(const 
     const unsigned sE0 = 8u * c0 + (((wb_abs + (unsigned)C::BOX_PHI) >> 7) << 4), sE1 = 8u * col1 + (((wb_abs + box1) >> 7) << 4);
     const unsigned sR1 = gam1 ? 3u : 13u;           // box rows per matrix row
     __syncthreads();
-    const double h6 = a.h / 6.0, hh = 0.5 * a.h;
+    const double h6 = a.rk.h6, hh = a.rk.an[0], h = a.rk.an[2];
     // Groups are claimed from a global counter instead of a fixed stride: warps that share a scheduler run at different
     // speeds, and a static split would leave the fast ones idle at the end.  The next group's input lines are pulled
     // into L2 while this one is computed (register free).
@@ -518,6 +557,8 @@ __global__ void __launch_bounds__(SfCfg<ARM>::WARPS * 32, 1) k_sens_fused(const 
             for (int c = 0; c < 3; ++c) u[c] = RIGID ? 0.0 : __ldcs(uin + (long)c * a.ld + ui);
 #pragma unroll
             for (int c = 0; c < 3; ++c) st_scratch(Sw + (13 + c) * 32 + lane, u[c]);     // (after ALL loads: may-alias stores serialise them)
+            // (not rk4_step: its peeled first stage puts a second copy of the RHS into this kernel's instruction stream,
+            // which made the kernel 1-4 % slower at 1 M units on a B200, 1000 W)
             NoSink ns;
 #pragma unroll 1
             for (int st = 0; st < 4; ++st) {
@@ -525,7 +566,7 @@ __global__ void __launch_bounds__(SfCfg<ARM>::WARPS * 32, 1) k_sens_fused(const 
                 for (int c = 0; c < 13; ++c) st_scratch(Sw + (st * 16 + c) * 32 + lane, xt[c]);
                 model_eval<RIGID, false>(a.K, a.K.A, xt, u, k, ns);
                 const double wgt = (st == 0 || st == 3) ? 1.0 : 2.0;
-                const double an = (st == 2) ? a.h : hh;
+                const double an = (st == 2) ? h : hh;
 #pragma unroll
                 for (int c = 0; c < 13; ++c) {
                     acc[c] = (st == 0) ? k[c] : fma(wgt, k[c], acc[c]);
@@ -593,38 +634,9 @@ __global__ void __launch_bounds__(SfCfg<ARM>::WARPS * 32, 1) k_sens_fused(const 
                 // ---- stages 2..4: S_i = [Jx_i | Ju_i] D_i, one copy of the code (rolled: instruction-cache footprint)
 #pragma unroll 1
                 for (int st = 1; st < 4; ++st) {
-                    const double* __restrict__ T = tile + p * C::PASS_S + st * C::TILE_S + C::at(0, lu);
-#pragma unroll
-                    for (int i = 0; i < 13; ++i) { N0[i] = 0.0; N1[i] = 0.0; }
-                    // column-major traversal: the (up to 13) entries J[i][j] of input row j update 26 independent chains
-                    // N[i][.], so consecutive DFMAs never depend on each other; columns 13..15 are the control seed
-                    // Operand order matters: a DFMA with three distinct vector-register operands issues every 3 cycles, with two
-                    // every 2 (profiles/r2j_dfma_operands.log).  The two FMAs of an entry share jv; alternating which column goes
-                    // first makes the first FMA of the NEXT entry share D[.][j] with the one before it, so that every FMA finds
-                    // one operand in the reuse cache: ... (D0, jv1) (D1, jv1) (D1, jv2) (D0, jv2) (D0, jv3) ...
-                    int flip = 0;
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) {
-#pragma unroll
-                        for (int i = (RIGID ? 6 : 0); i < 13; ++i) {
-                            if ((j < 13) ? jx_nz(i, j, ARM) : (!RIGID && ju_nz(i, j - 13))) {
-                                const double jv = T[SENS_TAB.col[i][j] * 2];     // broadcast LDS.64, immediate offset
-                                // the control rows of the seed are 0 for this lane's first column (c0 < 8) and e_(c1) for its second
-                                if (j >= 13) {
-                                    N1[i] = fma(jv, D[1][j], N1[i]);
-                                } else if (flip) {
-                                    N1[i] = fma(jv, D[1][j], N1[i]);
-                                    N0[i] = fma(jv, D[0][j], N0[i]);
-                                } else {
-                                    N0[i] = fma(jv, D[0][j], N0[i]);
-                                    N1[i] = fma(jv, D[1][j], N1[i]);
-                                }
-                                flip ^= 1;
-                            }
-                        }
-                    }
+                    jac_times2<ARM, RIGID, 2>(tile + p * C::PASS_S + st * C::TILE_S + C::at(0, lu), D[0], D[1], N0, N1);
                     const double wgt = (st == 3) ? 1.0 : 2.0;
-                    const double an = (st == 2) ? a.h : hh;
+                    const double an = (st == 2) ? h : hh;
 #pragma unroll
                     for (int i = 0; i < 13; ++i) {
                         A0[i] = fma(wgt, N0[i], A0[i]);
@@ -732,27 +744,6 @@ struct SmemSink {       // compact slots of this lane's filter in the warp's sha
     __device__ __forceinline__ void aero(double, double, double) const {}
 };
 
-// y[i] += sum_j J[i][j] v[j] for two vectors at once, J from the shared tile column of this lane's filter
-template <bool ARM, bool RIGID, int STRIDE = 4>      // STRIDE: filters per tile row ([slot][STRIDE])
-__device__ __forceinline__ void ekf_jx_times2(const double* __restrict__ T, const double (&v0)[13], const double (&v1)[13],
-                                              double (&y0)[13], double (&y1)[13]) {
-#pragma unroll
-    for (int i = 0; i < 13; ++i) { y0[i] = 0.0; y1[i] = 0.0; }
-    int flip = 0;           // alternate the order inside the pairs: every FMA then shares an operand with its predecessor (see k_sens_fused)
-#pragma unroll
-    for (int j = 0; j < 13; ++j) {
-#pragma unroll
-        for (int i = (RIGID ? 6 : 0); i < 13; ++i) {
-            if (jx_nz(i, j, ARM)) {
-                const double jv = T[SENS_TAB.jx[i][j] * STRIDE];
-                if (flip) { y1[i] = fma(jv, v1[j], y1[i]); y0[i] = fma(jv, v0[j], y0[i]); }
-                else { y0[i] = fma(jv, v0[j], y0[i]); y1[i] = fma(jv, v1[j], y1[i]); }
-                flip ^= 1;
-            }
-        }
-    }
-}
-
 // W (13 x 13 row-major) -> shared memory, one copy per CTA (the caller synchronises the block).  The kernel passes
 // threadIdx.x: read there, its range comes from the kernel's launch bounds, and with at most 169 threads the compiler
 // drops the loop's entry test.
@@ -767,34 +758,23 @@ __device__ __forceinline__ long ekf_claim_group(unsigned long long* next_group, 
     return (long)__shfl_sync(0xffffffffu, g, 0);
 }
 
-// The filter step of both predict kernels, one filter `unit` per lane: ONE evaluation of f and d f/d x at the pre-step state
-// gives the Jacobian (into `sink`) AND the first RK4 stage k1 (the reference evaluates both at the same point,
-// kiteEKF.cpp:80,93); `after_k1()` runs next, then three more RHS evaluations finish the step -> xn and the status word.
+// The filter step of both predict kernels, one filter `unit` per lane: the RK4 step's first stage evaluates f and d f/d x
+// at the pre-step state in ONE pass, giving the Jacobian (into `sink`) AND k1 (the reference evaluates both at the same
+// point, kiteEKF.cpp:80,93); `after_k1()` runs next, then three more RHS evaluations finish the step -> xn and the status word.
 // Ragged tail: lanes past B recompute the last filter and store nothing.
 template <bool RIGID, class Sink, class AfterK1>
 __device__ __forceinline__ void ekf_filter_step(const EkfArgs& a, long unit, Sink sink, AfterK1&& after_k1) {
     const long ui = unit < a.B ? unit : a.B - 1;
-    double x[13], u[3], k[13], acc[13], xt[13];
+    double x[13], u[3];
 #pragma unroll
     for (int c = 0; c < 13; ++c) x[c] = __ldcs(a.x + (long)c * a.ld + ui);
 #pragma unroll
     for (int c = 0; c < 3; ++c) u[c] = a.u ? __ldcs(a.u + (long)c * a.ld + ui) : 0.0;
     const int pre = a.status ? singularity_flags<RIGID>(x) : 0;
-    model_eval<RIGID, true>(a.K, a.K.A, x, u, k, sink);
-#pragma unroll
-    for (int c = 0; c < 13; ++c) { acc[c] = k[c]; xt[c] = fma(a.rk.an[0], k[c], x[c]); }
-    after_k1();
-    NoSink ns;
-#pragma unroll 1
-    for (int st = 1; st < 4; ++st) {
-        model_eval<RIGID, false>(a.K, a.K.A, xt, u, k, ns);
-        const double wgt = a.rk.w[st], an = a.rk.an[st];
-#pragma unroll
-        for (int c = 0; c < 13; ++c) { acc[c] = fma(wgt, k[c], acc[c]); xt[c] = fma(an, k[c], x[c]); }
-    }
+    rk4_step<RIGID, true>(a.K, a.K.A, x, u, a.rk, sink, [&](int st, const double (&)[13]) { if (st == 1) after_k1(); });
     if (unit < a.B) {
 #pragma unroll
-        for (int c = 0; c < 13; ++c) { x[c] = fma(a.rk.h6, acc[c], x[c]); __stcs(a.xn + (long)c * a.ld + unit, x[c]); }
+        for (int c = 0; c < 13; ++c) __stcs(a.xn + (long)c * a.ld + unit, x[c]);
         if (a.status) a.status[unit] = pre | (all_finite13(x) ? 0 : FLAG_NONFINITE);
     }
 }
@@ -841,7 +821,7 @@ __global__ void __launch_bounds__(EfCfg<ARM>::WARPS * 32, 1) k_ekf_predict(const
 #pragma unroll
             for (int k = 0; k < 13; ++k) { p0[k] = pn0[k]; p1[k] = pn1[k]; }
             if (p < 7) load_rows(g, p + 1, pn0, pn1);
-            ekf_jx_times2<ARM, RIGID>(T, p0, p1, n0, n1);
+            jac_times2<ARM, RIGID, 4>(T, p0, p1, n0, n1);
             __syncwarp();                               // the previous pass is done reading the transpose buffer
 #pragma unroll
             for (int k = 0; k < 13; ++k) {              // rows r0, r1 of Q = P A^T
@@ -854,7 +834,7 @@ __global__ void __launch_bounds__(EfCfg<ARM>::WARPS * 32, 1) k_ekf_predict(const
                 p0[k] = v0 ? Q[k * C::QR + r0] : 0.0;
                 p1[k] = v1 ? Q[k * C::QR + r1] : 0.0;
             }
-            ekf_jx_times2<ARM, RIGID>(T, p0, p1, n0, n1);
+            jac_times2<ARM, RIGID, 4>(T, p0, p1, n0, n1);
             if (unit < a.B) {
 #pragma unroll
                 for (int i = 0; i < 13; ++i) {          // columns r0, r1 of Pn = A Q + W
@@ -1028,7 +1008,7 @@ __global__ void __launch_bounds__(EtCfg<ARM>::WARPS * 32, 1) k_ekf_predict_tma(c
                     p0[k] = BX(row0 + k * 64u);
                     p1[k] = v1 ? BX(row1 + k * 64u) : 0.0;
                 }
-                ekf_jx_times2<ARM, RIGID, 8>(T, p0, p1, n0, n1);
+                jac_times2<ARM, RIGID, 8>(T, p0, p1, n0, n1);
 #pragma unroll
                 for (int k = 0; k < 13; ++k) {          // rows r0, r1 of Q = P A^T, in place
                     BX(row0 + k * 64u) = fma(a.dt, n0[k], p0[k]);
@@ -1041,7 +1021,7 @@ __global__ void __launch_bounds__(EtCfg<ARM>::WARPS * 32, 1) k_ekf_predict_tma(c
                     p0[k] = BX(col0 + k * (13 * 64u));
                     p1[k] = v1 ? BX(col1 + k * (13 * 64u)) : 0.0;
                 }
-                ekf_jx_times2<ARM, RIGID, 8>(T, p0, p1, n0, n1);
+                jac_times2<ARM, RIGID, 8>(T, p0, p1, n0, n1);
 #pragma unroll
                 for (int i = 0; i < 13; ++i) {          // columns r0, r1 of Pn = A Q + W, in place
                     BX(col0 + i * (13 * 64u)) = fma(a.dt, n0[i], p0[i]) + Ws[i * 13 + r0];

@@ -576,9 +576,14 @@ __host__ __device__ inline RkTab make_rk_tab(double h) {
     t.h6 = h / 6.0;
     return t;
 }
-template <bool RIGID, class AC>
+struct NoHook {
+    __device__ __forceinline__ void operator()(int, const double (&)[13]) const {}
+};
+// JAC: stage 1 also emits d f/d x and d f/d u at the pre-step state through `sink`.  `hook(st, xs)` runs before stage st
+// (0..3) with that stage's input state xs.
+template <bool RIGID, bool JAC = false, class AC, class Sink = NoSink, class Hook = NoHook>
 __device__ __forceinline__ void rk4_step(const KiteConsts& K, const AC& A, double (&x)[13], const double (&u)[3],
-                                         const RkTab& rk) {
+                                         const RkTab& rk, const Sink& sink = Sink{}, const Hook& hook = Hook{}) {
     NoSink ns;
     double k[13], acc[13], xt[13];
     const CtrlTerms uc = ctrl_terms(K, A, u);                    // the control is held for all four stages
@@ -587,11 +592,13 @@ __device__ __forceinline__ void rk4_step(const KiteConsts& K, const AC& A, doubl
     // result).  Stages 2..4 run as a real loop (one more copy of the RHS in the instruction stream: the fully unrolled body was
     // ~100 KB of SASS and stalled on instruction fetch, profiles/r1a_rollout_ncu_summary.txt; two copies do not).
     // Config 2: 77.8 -> 75.6 ms.
-    model_eval_c<RIGID, false>(K, A, x, uc, k, ns);
+    hook(0, x);
+    model_eval_c<RIGID, JAC>(K, A, x, uc, k, sink);
 #pragma unroll
     for (int i = 0; i < 13; ++i) { acc[i] = k[i]; xt[i] = fma(rk.an[0], k[i], x[i]); }
 #pragma unroll 1
     for (int st = 1; st < 4; ++st) {
+        hook(st, xt);
         model_eval_c<RIGID, false>(K, A, xt, uc, k, ns);
         const double wgt = rk.w[st];                             // tableau weights b = (1,2,2,1)/6
         const double an = rk.an[st];                             // next stage offset a = (1/2, 1/2, 1, 0)
